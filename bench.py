@@ -2,6 +2,7 @@
 """bench.py -- SSIMULACRA2 frame-pairs/s on B200 (BASELINE.json metric), one JSON line on stdout.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload 4k|1080p|512|1080p_srgb8] [--impl ours|reference]
+                  [--dump-outputs DIR]
   N > 1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
           (or, one process for all GPUs through the C ABI's own sharding: python bench.py --gpus N --shard-api)
 
@@ -229,10 +230,11 @@ def parity_block(norms_gpu, score_gpu, o_score, o_norms, what):
     return p
 
 
-def measure(c, workload, steps, warmup, batch, ring, e2e_steps, with_clocks=True, score_only=None):
+def measure(c, workload, steps, warmup, batch, ring, e2e_steps, with_clocks=True, score_only=None, outputs=False):
     """One workload on this rank's GPU: device-resident throughput, e2e from pinned host buffers + the raw H2D rate, per-kernel
     device times (ring = 1), the first pair's score + norms.  Returns a dict (times are max over ranks).
-    e2e_steps = 0 skips the host-buffer legs (used for the score-only sub-result, whose e2e is the same PCIe-bound figure)."""
+    e2e_steps = 0 skips the host-buffer legs (used for the score-only sub-result, whose e2e is the same PCIe-bound figure).
+    outputs = True also returns the scores and (outside score-only mode) the norms of every pair of the last timed step."""
     score_only = c.args.score_only if score_only is None else score_only
     torch, tm, synth, dist = c.torch, c.tm, c.synth, c.dist
     w, h, kind, bits, desc = WORKLOADS[workload]
@@ -281,7 +283,7 @@ def measure(c, workload, steps, warmup, batch, ring, e2e_steps, with_clocks=True
             if prev is not None:
                 m.get_scores(prev)
             prev = ts
-        m.get_scores(prev)
+        timed.tickets, timed.scores = prev, m.get_scores(prev)
         # get_scores() has synchronised every batch stream with the host; mark the end on the device clock
         e1.record(stream)
         torch.cuda.synchronize()
@@ -310,6 +312,13 @@ def measure(c, workload, steps, warmup, batch, ring, e2e_steps, with_clocks=True
     clocks = sampler.stop() if sampler else None
     launches = m.info().kernel_launches - l0
     value = c.world * n_pairs * steps / (ms / 1000.0)
+    last_step = None
+    if outputs:
+        import numpy as np
+        last_step = {"scores": timed.scores}
+        if not score_only:
+            # the library keeps the results of its last 16384 tickets on the host: no device work after the timed region
+            last_step["norms"] = np.stack([m.get_norms(t) for t in timed.tickets])
 
     e2e = None
     # ---- e2e: host frames through the C ABI, and the raw H2D rate of the same buffers (no kernels) for comparison
@@ -365,7 +374,8 @@ def measure(c, workload, steps, warmup, batch, ring, e2e_steps, with_clocks=True
     return {"workload": workload, "desc": desc, "w": w, "h": h, "kind": kind, "bits": bits, "value": value, "ms": ms, "steps": steps,
             "warmup": warmup, "timing": timing, "clocks": clocks, "launches": int(launches), "e2e": e2e, "info": info,
             "frame_bytes": frame_bytes, "n_pairs": n_pairs, "n_distinct": n_distinct, "kms": kms, "kbatches": kbatches, "kpairs": kpairs,
-            "s_first": s_first, "s_last": s_last, "norms_first": norms_first, "pitch": pitch, "ch": ch}
+            "s_first": s_first, "s_last": s_last, "norms_first": norms_first, "pitch": pitch, "ch": ch,
+            "last_step": last_step}
 
 
 def roofline_block(c, r):
@@ -481,6 +491,8 @@ def run_shard_api(args):
         sampler = ClockSampler(0).start()
         dt, sc = run(lambda: sh.submit_device(refs, diss), args.steps)
         clocks = sampler.stop()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"scores": sc})
         run(lambda: sh.submit_host(hrefs, hdiss), 1)
         e2e_steps = max(1, min(args.steps, 2))
         dt_h, sc_h = run(lambda: sh.submit_host(hrefs, hdiss), e2e_steps)
@@ -521,7 +533,10 @@ def run_ours(args, rank, world, local_rank):
     workload = args.workload
     w, h, kind, bits, desc = WORKLOADS[workload]
     batch = args.batch or BATCH[workload]
-    r = measure(c, workload, args.steps, args.warmup, batch, args.ring, max(1, min(args.steps, 3)))
+    r = measure(c, workload, args.steps, args.warmup, batch, args.ring, max(1, min(args.steps, 3)), outputs=bool(args.dump_outputs))
+    if args.dump_outputs:
+        suffix = "" if world == 1 else f"_rank{rank}"
+        dump_outputs(args.dump_outputs, {k + suffix: v for k, v in r["last_step"].items()})
 
     # ---- the other BASELINE configs, measured in the same run (fewer steps: they are sub-results, not the headline)
     subs = {}
@@ -635,6 +650,15 @@ def run_ours(args, rank, world, local_rank):
     emit(line)
 
 
+def dump_outputs(d, arrays):
+    """Writes each array as d/<name>.npy in float64.  The inputs are seeded, so two builds run with the same arguments
+    can be compared output for output."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 _REAL_STDOUT = None
 
 
@@ -671,7 +695,14 @@ def main():
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-refgpu", action="store_true", help="skip the reference-design GPU baseline (baseline/refgpu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the scores of the last timed step to DIR/scores.npy and, "
+                    "except with --score-only or --shard-api, their 108 norms each to DIR/norms.npy "
+                    "(DIR/<name>_rank<r>.npy per rank under torchrun)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; --impl reference has no GPU path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -95,10 +95,14 @@ def downscale(lin):
     return 0.25 * (p[:, 0::2, 0::2] + p[:, 0::2, 1::2] + p[:, 1::2, 0::2] + p[:, 1::2, 1::2])
 
 
+# opsin absorbance matrix and bias of the SSIMULACRA2 definition (cpu.rs:421-470), f64
+OPSIN_M = np.array([[0.30, 0.622, 0.078], [0.23, 0.692, 0.078], [0.24342268924547819, 0.20476744424496821, 0.55180986650955360]])
+OPSIN_BIAS = 0.0037930732552754493
+
+
 def xyb(lin):
     """Opsin absorbance -> cube root -> XYB, rescaled positive (cpu.rs:421-496), f64."""
-    m = np.array([[0.30, 0.622, 0.078], [0.23, 0.692, 0.078], [0.24342268924547819, 0.20476744424496821, 0.55180986650955360]])
-    bias = 0.0037930732552754493
+    m, bias = OPSIN_M, OPSIN_BIAS
     mixed = np.maximum(np.tensordot(m, lin, axes=(1, 0)) + bias, 0.0)
     t = np.cbrt(mixed) - np.cbrt(bias)
     x, y = 0.5 * (t[0] - t[1]), 0.5 * (t[0] + t[1])
@@ -281,6 +285,21 @@ def test_fir_taps_match_the_documented_kernel():
     assert np.allclose(mul_in, [0.055295236, -0.058836687, 0.012955819], rtol=1e-6)        # cpu.rs:931-948
     assert np.allclose(mul_prev, [1.9021131, 1.1755705, 1.2246469e-16], rtol=1e-6)
     assert np.allclose(taps[4:], [0.264621, 0.212929, 0.109335, 0.036011, 0.009414], atol=1e-6)   # SURVEY.md 8(a7)
+
+
+def test_oracle_filter_and_opsin_constants_are_the_f32_roundings_of_their_definitions(oracle):
+    """Bit for bit: the oracle's recursive-filter constants are the f32 roundings of the f64 values derived in
+    gaussian_taps() (MUL_PREV2 = -1), and its opsin constants are the f32 roundings of OPSIN_M / OPSIN_BIAS, with each
+    row's middle entry (last entry for the third row) formed as 1 - the other two in f32 and the bias's cube root rounded
+    once from f64."""
+    f = np.float32
+    _, mul_in, mul_prev = gaussian_taps()
+    expect = np.concatenate([mul_in, mul_prev, np.full(3, -1.0, f)])
+    assert np.array_equal(oracle.rg_constants().view(np.uint32), expect.view(np.uint32))
+    m = OPSIN_M.astype(f)
+    expect = np.array([m[0, 0], f(1) - m[0, 2] - m[0, 0], m[0, 2], m[1, 0], f(1) - m[1, 2] - m[1, 0], m[1, 2],
+                       m[2, 0], m[2, 1], f(1) - m[2, 0] - m[2, 1], f(OPSIN_BIAS), f(np.cbrt(OPSIN_BIAS)), 0], f)
+    assert np.array_equal(oracle.opsin_constants().view(np.uint32), expect.view(np.uint32))
 
 
 def _both(oracle, name, kind, args):
