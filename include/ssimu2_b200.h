@@ -5,6 +5,8 @@
  * that feeds it (paths relative to /root/reference/crates):
  *
  *   ssimulacra2-cuda/src/lib.rs:27-107   struct Ssimulacra2 / Ssimulacra2::new      -> ssimu2_create
+ *   turbo-metrics/src/lib.rs:268-360     compute_one(fref, cc_ref, fdis, cc_dis)    -> ssimu2_create_mixed when the two
+ *                                        sources differ in HwFrame variant or colour characteristics
  *   ssimulacra2-cuda/src/lib.rs:110      Ssimulacra2::mem_usage                     -> ssimu2_mem_usage
  *   ssimulacra2-cuda/src/lib.rs:283-287  Ssimulacra2::compute (async)               -> ssimu2_submit
  *   ssimulacra2-cuda/src/lib.rs:271-279  Ssimulacra2::compute_sync                  -> ssimu2_compute_sync
@@ -42,6 +44,9 @@
  *     target named by BASELINE.json is the CPU implementation.  ssimu2_info.nscales tells which case applies.
  *   - A handle is bound to one device and one (width, height, format).  Calls on one handle
  *     are not re-entrant; different handles may be driven from different threads.
+ *   - Mixed sources: ssimu2_create_mixed binds the distorted frames to a description of their own (format, matrix, range),
+ *     like TurboMetrics::compute_one(fref, cc_ref, fdis, cc_dis), which converts each frame with its own HwFrame variant and
+ *     colour characteristics (turbo-metrics/src/lib.rs:268-360).  Both sides keep one width and height.
  *   - There is no CPU fallback: if no CUDA device is usable every entry point fails.
  */
 #ifndef SSIMU2_B200_H
@@ -120,8 +125,25 @@ typedef struct {
     uint32_t reserved[5]; /* must be 0 */
 } ssimu2_config;
 
+/* The description of the DISTORTED frames of a mixed handle (ssimu2_create_mixed); ssimu2_config describes the reference. */
+typedef struct {
+    int32_t format;       /* ssimu2_format of the distorted frames */
+    int32_t matrix;       /* ssimu2_matrix (YUV formats) */
+    int32_t full_range;   /* 0 = limited, 1 = full */
+    uint32_t flags;       /* SSIMU2_FLAG_P016_DEEP only, and only with format == SSIMU2_FMT_P016 */
+    uint32_t reserved[4]; /* must be 0 */
+} ssimu2_source;
+
 /* ---- lifetime ------------------------------------------------------------------------ */
 int ssimu2_create(ssimu2_t **out, const ssimu2_config *cfg);
+/* A handle whose distorted frames have their own pixel format / matrix / range.  cfg describes the reference frames (its
+ * SSIMU2_FLAG_P016_DEEP applies to the reference side only); dis == NULL: exactly ssimu2_create.  `dis` is checked before any
+ * device call: a bad format or matrix, a flag other than SSIMU2_FLAG_P016_DEEP, or that flag with a format other than P016 is
+ * SSIMU2_E_UNSUPPORTED; non-zero reserved fields are SSIMU2_E_INVALID.  When the two sides are the same effective description
+ * (same format and deep flag; for NV12 / P016 also the same matrix and range) the result is an ordinary handle: one
+ * front-end launch per input group and the same bits.  Otherwise the front-end runs once per side on the slot's stream, and
+ * the frames of each side are checked against that side's format (ssimu2_frame pitch rule). */
+int ssimu2_create_mixed(ssimu2_t **out, const ssimu2_config *cfg, const ssimu2_source *dis);
 int ssimu2_destroy(ssimu2_t *h);
 /* Device bytes owned by the handle (Ssimulacra2::mem_usage). */
 int ssimu2_mem_usage(const ssimu2_t *h, size_t *bytes);
@@ -177,6 +199,12 @@ int ssimu2_submit_host(ssimu2_t *h, const ssimu2_frame *ref, const ssimu2_frame 
  * decodes on the CPU (turbo-metrics/src/input_image.rs:206-228 copies each frame itself) becomes one call per chunk. */
 int ssimu2_submit_host_batch(ssimu2_t *h, uint32_t n, const ssimu2_frame *refs, const ssimu2_frame *diss,
                              size_t frame_bytes, uint64_t *first_ticket);
+/* Host frames whose two sides have different sizes (a mixed handle, e.g. an NV12 reference against a P016 encode): reference i
+ * copies ref_bytes starting at refs[i].plane[0], distorted i copies dis_bytes.  Otherwise as ssimu2_submit_host_batch, which
+ * (like ssimu2_submit_host) is this call with ref_bytes == dis_bytes and returns SSIMU2_E_INVALID on a mixed handle whose
+ * two sides have different bytes per pixel. */
+int ssimu2_submit_host_sized(ssimu2_t *h, uint32_t n, const ssimu2_frame *refs, size_t ref_bytes, const ssimu2_frame *diss,
+                             size_t dis_bytes, uint64_t *first_ticket);
 
 /* ---- results on the device ----------------------------------------------------------- */
 /* Device address of the f64 score ring (one entry per ticket, index ticket % capacity). */
@@ -205,11 +233,17 @@ int ssimu2_get_info(const ssimu2_t *h, ssimu2_info *info);
 typedef struct ssimu2_shard ssimu2_shard_t;
 /* cfg->device is ignored; devices[i] are CUDA ordinals (n_devices >= 1). */
 int ssimu2_shard_create(ssimu2_shard_t **out, const ssimu2_config *cfg, const int32_t *devices, uint32_t n_devices);
+/* Every worker's handle is ssimu2_create_mixed(cfg, dis); dis == NULL: ssimu2_shard_create. */
+int ssimu2_shard_create_mixed(ssimu2_shard_t **out, const ssimu2_config *cfg, const ssimu2_source *dis, const int32_t *devices,
+                              uint32_t n_devices);
 int ssimu2_shard_destroy(ssimu2_shard_t *s);
 /* n host pairs (layout as ssimu2_submit_host); returns at once, the copies and launches run on the worker threads.
  * The frames must stay valid until their scores have been fetched.  *first_ticket = global ticket of pair 0. */
 int ssimu2_shard_submit_host(ssimu2_shard_t *s, uint32_t n, const ssimu2_frame *refs, const ssimu2_frame *diss,
                              size_t frame_bytes, uint64_t *first_ticket);
+/* Host pairs with one byte count per side (layout as ssimu2_submit_host_sized); otherwise as ssimu2_shard_submit_host. */
+int ssimu2_shard_submit_host_sized(ssimu2_shard_t *s, uint32_t n, const ssimu2_frame *refs, size_t ref_bytes,
+                                   const ssimu2_frame *diss, size_t dis_bytes, uint64_t *first_ticket);
 /* n DEVICE pairs that already live on the GPU the sharding rule assigns them to (ssimu2_shard_device_of); `streams[d]`
  * (may be NULL = no dependency) is the stream of device d the frames were produced on. */
 int ssimu2_shard_submit_device(ssimu2_shard_t *s, uint32_t n, const ssimu2_frame *refs, const ssimu2_frame *diss,

@@ -26,6 +26,12 @@ class Config(C.Structure):
                 ("input_group", C.c_uint32), ("reserved", C.c_uint32 * 5)]
 
 
+class Source(C.Structure):
+    """ssimu2_source: the description of the distorted frames of a mixed handle (ssimu2_create_mixed)."""
+    _fields_ = [("format", C.c_int32), ("matrix", C.c_int32), ("full_range", C.c_int32), ("flags", C.c_uint32),
+                ("reserved", C.c_uint32 * 4)]
+
+
 PIPELINE_DEFAULT, PIPELINE_SPLIT = 0, 1
 FLAG_SCORE_ONLY, FLAG_NO_TIMING, FLAG_P016_DEEP = 1, 2, 4
 
@@ -44,6 +50,7 @@ _P = C.c_void_p
 _FP = C.POINTER(Frame)
 SYMBOLS = {
     "ssimu2_create": (C.c_int, [C.POINTER(_P), C.POINTER(Config)]),
+    "ssimu2_create_mixed": (C.c_int, [C.POINTER(_P), C.POINTER(Config), C.POINTER(Source)]),
     "ssimu2_destroy": (C.c_int, [_P]),
     "ssimu2_mem_usage": (C.c_int, [_P, C.POINTER(C.c_size_t)]),
     "ssimu2_strerror": (C.c_char_p, [C.c_int]),
@@ -61,6 +68,7 @@ SYMBOLS = {
     "ssimu2_stream_wait_input": (C.c_int, [_P, C.c_uint64, _P]),
     "ssimu2_submit_host": (C.c_int, [_P, _FP, _FP, C.c_size_t, C.POINTER(C.c_uint64)]),
     "ssimu2_submit_host_batch": (C.c_int, [_P, C.c_uint32, _FP, _FP, C.c_size_t, C.POINTER(C.c_uint64)]),
+    "ssimu2_submit_host_sized": (C.c_int, [_P, C.c_uint32, _FP, C.c_size_t, _FP, C.c_size_t, C.POINTER(C.c_uint64)]),
     "ssimu2_scores_device": (C.c_int, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "ssimu2_get_info": (C.c_int, [_P, C.POINTER(Info)]),
     "ssimu2_debug_read": (C.c_int, [_P, C.c_uint64, C.c_int, C.c_int, C.POINTER(C.c_float), C.c_size_t]),
@@ -68,8 +76,11 @@ SYMBOLS = {
     "ssimu2_last_batch_ms": (C.c_int, [_P, C.POINTER(C.c_float)]),
     "ssimu2_kernel_ms": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int]),
     "ssimu2_shard_create": (C.c_int, [C.POINTER(_P), C.POINTER(Config), C.POINTER(C.c_int32), C.c_uint32]),
+    "ssimu2_shard_create_mixed": (C.c_int, [C.POINTER(_P), C.POINTER(Config), C.POINTER(Source), C.POINTER(C.c_int32),
+                                            C.c_uint32]),
     "ssimu2_shard_destroy": (C.c_int, [_P]),
     "ssimu2_shard_submit_host": (C.c_int, [_P, C.c_uint32, _FP, _FP, C.c_size_t, C.POINTER(C.c_uint64)]),
+    "ssimu2_shard_submit_host_sized": (C.c_int, [_P, C.c_uint32, _FP, C.c_size_t, _FP, C.c_size_t, C.POINTER(C.c_uint64)]),
     "ssimu2_shard_submit_device": (C.c_int, [_P, C.c_uint32, _FP, _FP, C.POINTER(_P), C.POINTER(C.c_uint64)]),
     "ssimu2_shard_device_of": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_int32)]),
     "ssimu2_shard_get_scores": (C.c_int, [_P, C.c_uint64, C.c_uint32, C.POINTER(C.c_double)]),

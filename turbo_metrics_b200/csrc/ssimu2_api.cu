@@ -85,7 +85,14 @@ struct Slot {
 
 struct ssimu2_handle {
     ssimu2_config cfg{};
-    Geo geo{};
+    Geo geo{};                        // geometry + the reference side's coefficients and memo table
+    // mixed sources (ssimu2_create_mixed with a distorted description that differs from cfg): the front-end runs once per
+    // side, the distorted side with geo_dis (geo with that side's coefficients and memo table)
+    bool mixed = false;
+    int fmt[2] = {0, 0};              // ssimu2_format of the reference / distorted frames
+    int fe_fmt[2] = {0, 0};           // their front-end formats (kP016A: P016 with SSIMU2_FLAG_P016_DEEP)
+    Geo geo_dis{};
+    float* eotf_lut_dis = nullptr;
     uint32_t batch = 0, ring = 0, input_group = 0;
     std::vector<Slot> slots;
     uint32_t cur = 0;
@@ -203,10 +210,65 @@ static void build_geo(ssimu2_handle* h)
     g.items_h = 0; g.items_v = 0;
     for (int s = 0; s < ns; s++) { g.items_h += g.sc[s].n_bands; g.items_v += g.sc[s].n_strips; }
     g.coef = make_coef(h->cfg.format, h->cfg.matrix, h->cfg.full_range);
-    // SURVEY.md section 8(d): B_alg = 120*sum(P_s) + 2*in_0*P_0 + 72*sum_{s>=1}(P_s)
-    h->alg_bytes = 120ULL * sum_px + 2ULL * in_bytes_per_px(h->cfg.format) * h->cfg.width * h->cfg.height + 72ULL * sum_px_ge1;
+    // SURVEY.md section 8(d): B_alg = 120*sum(P_s) + 2*in_0*P_0 + 72*sum_{s>=1}(P_s), in_0 = input bytes per pixel of the pair
+    // (each side at its own bytes per pixel: in_bytes_per_px is per two images of one format)
+    const unsigned long long in2 = (unsigned long long)(in_bytes_per_px(h->fmt[0]) + in_bytes_per_px(h->fmt[1]));
+    h->alg_bytes = 120ULL * sum_px + in2 * h->cfg.width * h->cfg.height + 72ULL * sum_px_ge1;
     // compulsory I/O floor B_io = in_0 * P_0 + 8
-    h->io_bytes = (unsigned long long)in_bytes_per_px(h->cfg.format) * h->cfg.width * h->cfg.height + 8ULL;
+    h->io_bytes = in2 * h->cfg.width * h->cfg.height / 2 + 8ULL;
+}
+
+// Exact memo of one side's transfer function (Geo::eotf_lut), built by the device code it replaces: the R / B tables of
+// 10-bit P016 and NV12, the sRGB16 table.  The other formats (and deep P016) have none.
+static cudaError_t build_side_lut(int fmt, bool deep, Geo& g, float** lut, size_t* bytes)
+{
+    *bytes = 0;
+    if ((fmt == kNV12 || fmt == kP016) && !deep) {
+        const int n = fmt == kNV12 ? 256 : 1024, shift = fmt == kNV12 ? 0 : 6;
+        const size_t b = (size_t)2 * n * n * sizeof(float);
+        cudaError_t e = cudaMalloc(lut, b);
+        if (e != cudaSuccess) return e;
+        k_build_eotf_lut<<<(n * n + 255) / 256, 256>>>(g.coef, n, shift, *lut);
+        if ((e = cudaGetLastError()) != cudaSuccess || (e = cudaDeviceSynchronize()) != cudaSuccess) return e;
+        g.eotf_lut = *lut;
+        g.lut_n = n;
+        g.lut_shift = shift;
+        *bytes = b;
+    }
+    if (fmt == kSRGB16) {
+        // exact memo of the sRGB16 transfer function: one gather per sample instead of one powf
+        const size_t b = (size_t)65536 * sizeof(float);
+        cudaError_t e = cudaMalloc(lut, b);
+        if (e != cudaSuccess) return e;
+        k_build_srgb16_lut<<<65536 / 256, 256>>>(*lut);
+        if ((e = cudaGetLastError()) != cudaSuccess || (e = cudaDeviceSynchronize()) != cudaSuccess) return e;
+        g.eotf_lut = *lut;
+        g.lut_n = 65536;
+        g.lut_shift = 0;
+        *bytes = b;
+    }
+    return cudaSuccess;
+}
+
+// the distorted description of ssimu2_create_mixed (checked like ssimu2_config, before any device call)
+static int check_source(const ssimu2_source* s)
+{
+    if (s->format < 0 || s->format > kLINEARF32) return SSIMU2_E_UNSUPPORTED;
+    if (s->matrix < 0 || s->matrix > 2) return SSIMU2_E_UNSUPPORTED;
+    if (s->flags & ~SSIMU2_FLAG_P016_DEEP) return SSIMU2_E_UNSUPPORTED;
+    if ((s->flags & SSIMU2_FLAG_P016_DEEP) && s->format != kP016) return SSIMU2_E_UNSUPPORTED;
+    for (int i = 0; i < 4; i++)
+        if (s->reserved[i]) return SSIMU2_E_INVALID;
+    return SSIMU2_OK;
+}
+
+// The two sides are one effective description: same format and deep flag, and (YUV) same matrix and range.  Matrix and range
+// mean nothing to the packed formats.
+static bool same_source(const ssimu2_config* cfg, const ssimu2_source* s)
+{
+    const bool yuv = cfg->format == kNV12 || cfg->format == kP016;
+    return s->format == cfg->format && (s->flags & SSIMU2_FLAG_P016_DEEP) == (cfg->flags & SSIMU2_FLAG_P016_DEEP) &&
+           (!yuv || (s->matrix == cfg->matrix && (s->full_range != 0) == (cfg->full_range != 0)));
 }
 
 // ---- TMA tensor maps (driver entry point fetched through the runtime; libcuda is not linked) ----
@@ -264,16 +326,32 @@ static int build_tma_maps(ssimu2_handle* h, Slot& sl)
 // All work of a batch runs on its slot's stream: [frame-table upload + front-end] x (1 .. n launches), then
 // k_hv + k_finalize (or k_hpass + k_vpass + k_finalize), then the D2H copy of scores and norms.
 
-template <int FMT>
-static void launch_frontend_kernel(const ssimu2_handle* h, Slot& sl, uint32_t frame0, uint32_t n)
+template <int FMT, int SIDE>
+static void launch_frontend_kernel(const Geo& g, Slot& sl, uint32_t frame0, uint32_t n)
 {
-    const Geo& g = h->geo;
     const int rx = (g.sc[0].w + kF2Region - 1) / kF2Region, ry = (g.sc[0].h + kF2Region - 1) / kF2Region;
-    const int per_cta = (kF2Threads / 32) * kF2RegionsPerWarp;
-    k_frontend2<FMT><<<dim3((rx + per_cta - 1) / per_cta, ry, n), kF2Threads, 0, sl.stream>>>(g, sl.in_d, sl.xyb, (int)frame0);
+    const int per_cta = (kF2Threads / 32) * f2_regions_per_warp(SIDE);
+    k_frontend2<FMT, SIDE><<<dim3((rx + per_cta - 1) / per_cta, ry, n), kF2Threads, 0, sl.stream>>>(g, sl.in_d, sl.xyb, (int)frame0);
 }
 
-// front-end of pairs [sl.fe_pairs, upto) of the batch being recorded in `sl`
+// fe_fmt: the front-end format of the side(s) (kP016A for P016 with SSIMU2_FLAG_P016_DEEP)
+template <int SIDE>
+static int launch_frontend_side(const Geo& g, int fe_fmt, Slot& sl, uint32_t frame0, uint32_t n)
+{
+    switch (fe_fmt) {
+    case kNV12: launch_frontend_kernel<kNV12, SIDE>(g, sl, frame0, n); break;
+    case kP016: launch_frontend_kernel<kP016, SIDE>(g, sl, frame0, n); break;
+    case kP016A: launch_frontend_kernel<kP016A, SIDE>(g, sl, frame0, n); break;
+    case kSRGB8: launch_frontend_kernel<kSRGB8, SIDE>(g, sl, frame0, n); break;
+    case kSRGB16: launch_frontend_kernel<kSRGB16, SIDE>(g, sl, frame0, n); break;
+    case kSRGBF32: launch_frontend_kernel<kSRGBF32, SIDE>(g, sl, frame0, n); break;
+    case kLINEARF32: launch_frontend_kernel<kLINEARF32, SIDE>(g, sl, frame0, n); break;
+    default: return SSIMU2_E_UNSUPPORTED;
+    }
+    return 0;
+}
+
+// front-end of pairs [sl.fe_pairs, upto) of the batch being recorded in `sl`: one launch, or on a mixed handle one per side
 static int launch_frontend(ssimu2_handle* h, Slot& sl, uint32_t upto, bool time_it)
 {
     const uint32_t f0 = sl.fe_pairs;
@@ -286,21 +364,18 @@ static int launch_frontend(ssimu2_handle* h, Slot& sl, uint32_t upto, bool time_
     }
     CU_TRY(cudaMemcpyAsync(sl.in_d + f0, sl.in_h + f0, (size_t)n * sizeof(FramePair), cudaMemcpyHostToDevice, sl.stream));
     if (time_it) cudaEventRecord(sl.ev_k[0], sl.stream);
-    switch (h->cfg.format) {
-    case kNV12: launch_frontend_kernel<kNV12>(h, sl, f0, n); break;
-    case kP016:
-        if (h->cfg.flags & SSIMU2_FLAG_P016_DEEP) launch_frontend_kernel<kP016A>(h, sl, f0, n);
-        else launch_frontend_kernel<kP016>(h, sl, f0, n);
-        break;
-    case kSRGB8: launch_frontend_kernel<kSRGB8>(h, sl, f0, n); break;
-    case kSRGB16: launch_frontend_kernel<kSRGB16>(h, sl, f0, n); break;
-    case kSRGBF32: launch_frontend_kernel<kSRGBF32>(h, sl, f0, n); break;
-    case kLINEARF32: launch_frontend_kernel<kLINEARF32>(h, sl, f0, n); break;
-    default: return SSIMU2_E_UNSUPPORTED;
+    int r;
+    if (!h->mixed) {
+        r = launch_frontend_side<kF2Both>(h->geo, h->fe_fmt[0], sl, f0, n);
+    } else {
+        r = launch_frontend_side<kF2Ref>(h->geo, h->fe_fmt[0], sl, f0, n);
+        if (!r) r = launch_frontend_side<kF2Dis>(h->geo_dis, h->fe_fmt[1], sl, f0, n);
     }
+    if (r) return r;
+    // the timing mark and the "inputs consumed" event follow the last launch: both sides have been read
     if (time_it) cudaEventRecord(sl.ev_k[1], sl.stream);
     CU_TRY(cudaGetLastError());
-    h->launches += 1;
+    h->launches += h->mixed ? 2 : 1;
     if (sl.fe_launches >= sl.ev_fe.size()) {
         cudaEvent_t e = nullptr;
         CU_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -422,13 +497,17 @@ static int finish_pair(ssimu2_handle* h)
     return 0;
 }
 
-static bool frame_ok(const ssimu2_handle* h, const ssimu2_frame* f)
+static bool is_yuv(int fmt) { return fmt == kNV12 || fmt == kP016; }
+
+// side 0: a reference frame, 1: a distorted frame (each side is checked against its own format)
+static bool frame_ok(const ssimu2_handle* h, const ssimu2_frame* f, int side)
 {
+    const int fmt = h->fmt[side];
     if (!f || !f->plane[0] || f->pitch == 0) return false;
-    if ((h->cfg.format == kNV12 || h->cfg.format == kP016) && !f->plane[1]) return false;
+    if (is_yuv(fmt) && !f->plane[1]) return false;
     // a row must fit in the pitch (rows that overlap would be read as garbage, and past the end of the last one)
     static const uint32_t bytes_per_px[] = {1, 2, 3, 6, 12, 12};   // NV12 / P016: per luma sample; packed RGB: per pixel
-    if ((uint64_t)f->pitch < (uint64_t)h->cfg.width * bytes_per_px[h->cfg.format]) return false;
+    if ((uint64_t)f->pitch < (uint64_t)h->cfg.width * bytes_per_px[fmt]) return false;
     return true;
 }
 
@@ -475,11 +554,50 @@ static int note_dependency(Slot& sl, void* stream)
     return 0;
 }
 
+// one host pair: copy each frame (its own byte count) to the slot's staging ring and record the pair
+static int submit_host_pair(ssimu2_handle* h, const ssimu2_frame* ref, size_t ref_bytes, const ssimu2_frame* dis, size_t dis_bytes)
+{
+    if (!frame_ok(h, ref, 0) || !frame_ok(h, dis, 1) || ref_bytes == 0 || dis_bytes == 0) return SSIMU2_E_INVALID;
+    const bool yuv_ref = is_yuv(h->fmt[0]), yuv_dis = is_yuv(h->fmt[1]);
+    if (yuv_ref && (ref->plane[1] <= ref->plane[0] || ref->plane[1] - ref->plane[0] >= ref_bytes)) return SSIMU2_E_INVALID;
+    if (yuv_dis && (dis->plane[1] <= dis->plane[0] || dis->plane[1] - dis->plane[0] >= dis_bytes)) return SSIMU2_E_INVALID;
+    DeviceGuard guard(h->cfg.device);
+    const size_t frame_bytes = ref_bytes > dis_bytes ? ref_bytes : dis_bytes;
+    if (frame_bytes > h->staging_frame_bytes) {
+        // (re)allocate the staging rings; rare (first call), so a full drain is acceptable
+        int fr = ssimu2_flush(h);
+        if (fr) return fr;
+        for (uint32_t i = 0; i < h->ring; i++) {
+            int r = harvest(h, i);
+            if (r) return r;
+        }
+        size_t fb = (frame_bytes + 255) / 256 * 256;
+        for (auto& sl : h->slots) {
+            cudaFree(sl.staging);
+            sl.staging = nullptr;
+            if (cudaMalloc(&sl.staging, fb * 2 * h->batch) != cudaSuccess) { cudaGetLastError(); return SSIMU2_E_NOMEM; }
+        }
+        h->device_bytes += (fb - h->staging_frame_bytes) * 2 * h->batch * h->ring;
+        h->staging_frame_bytes = fb;
+    }
+    int r = prepare_cur(h);
+    if (r) return r;
+    Slot& sl = h->slots[h->cur];
+    uint8_t* da = sl.staging + (size_t)(2 * sl.count) * h->staging_frame_bytes;
+    uint8_t* db = da + h->staging_frame_bytes;
+    CU_TRY(cudaMemcpyAsync(da, (const void*)ref->plane[0], ref_bytes, cudaMemcpyHostToDevice, sl.stream));
+    CU_TRY(cudaMemcpyAsync(db, (const void*)dis->plane[0], dis_bytes, cudaMemcpyHostToDevice, sl.stream));
+    FramePair& fp = sl.in_h[sl.count];
+    fp.ref.p0 = da; fp.ref.p1 = yuv_ref ? da + (ref->plane[1] - ref->plane[0]) : nullptr; fp.ref.pitch = ref->pitch; fp.ref.pad = 0;
+    fp.dis.p0 = db; fp.dis.p1 = yuv_dis ? db + (dis->plane[1] - dis->plane[0]) : nullptr; fp.dis.pitch = dis->pitch; fp.dis.pad = 0;
+    return finish_pair(h);
+}
+
 }  // namespace
 
 extern "C" {
 
-uint32_t ssimu2_version(void) { return (2u << 16) | 0u; }
+uint32_t ssimu2_version(void) { return (2u << 16) | 1u; }
 
 const char* ssimu2_strerror(int status)
 {
@@ -496,7 +614,9 @@ const char* ssimu2_strerror(int status)
     return "unknown status";
 }
 
-int ssimu2_create(ssimu2_t** out, const ssimu2_config* cfg)
+int ssimu2_create(ssimu2_t** out, const ssimu2_config* cfg) { return ssimu2_create_mixed(out, cfg, nullptr); }
+
+int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_source* dis)
 {
     if (!out || !cfg) return SSIMU2_E_INVALID;
     *out = nullptr;
@@ -509,6 +629,10 @@ int ssimu2_create(ssimu2_t** out, const ssimu2_config* cfg)
     if ((cfg->flags & SSIMU2_FLAG_SCORE_ONLY) && cfg->pipeline != SSIMU2_PIPELINE_DEFAULT) return SSIMU2_E_UNSUPPORTED;
     for (int i = 0; i < 5; i++)
         if (cfg->reserved[i]) return SSIMU2_E_INVALID;
+    if (dis) {
+        const int rc = check_source(dis);
+        if (rc) return rc;
+    }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
         cudaGetLastError();
@@ -523,6 +647,13 @@ int ssimu2_create(ssimu2_t** out, const ssimu2_config* cfg)
     ssimu2_handle* h = new (std::nothrow) ssimu2_handle();
     if (!h) return SSIMU2_E_NOMEM;
     h->cfg = *cfg;
+    h->mixed = dis != nullptr && !same_source(cfg, dis);
+    const bool deep_ref = (cfg->flags & SSIMU2_FLAG_P016_DEEP) != 0;
+    const bool deep_dis = h->mixed ? (dis->flags & SSIMU2_FLAG_P016_DEEP) != 0 : deep_ref;
+    h->fmt[0] = cfg->format;
+    h->fmt[1] = h->mixed ? dis->format : cfg->format;
+    h->fe_fmt[0] = deep_ref ? kP016A : h->fmt[0];
+    h->fe_fmt[1] = deep_dis ? kP016A : h->fmt[1];
     h->ring = cfg->ring ? cfg->ring : kDefaultRing;
     if (h->ring > 16) h->ring = 16;
     h->batch = cfg->batch ? cfg->batch : kDefaultBatch;
@@ -583,28 +714,19 @@ int ssimu2_create(ssimu2_t** out, const ssimu2_config* cfg)
         for (int i = 0; i < 256; i++) cs.tab[i] = exact_math::cbrt_scale_entry(i);
         CR(cudaMemcpyToSymbol(kCbrtC, &cs, sizeof(cs)));
     }
-    if ((cfg->format == kNV12 || cfg->format == kP016) && !(cfg->flags & SSIMU2_FLAG_P016_DEEP)) {
-        const int n = cfg->format == kNV12 ? 256 : 1024, shift = cfg->format == kNV12 ? 0 : 6;
-        const size_t bytes = (size_t)2 * n * n * sizeof(float);
-        CR(cudaMalloc(&h->eotf_lut, bytes));
-        k_build_eotf_lut<<<(n * n + 255) / 256, 256>>>(h->geo.coef, n, shift, h->eotf_lut);
-        CR(cudaGetLastError());
-        CR(cudaDeviceSynchronize());
-        h->geo.eotf_lut = h->eotf_lut;
-        h->geo.lut_n = n;
-        h->geo.lut_shift = shift;
+    {
+        size_t bytes = 0;
+        CR(build_side_lut(h->fmt[0], deep_ref, h->geo, &h->eotf_lut, &bytes));
         h->device_bytes += bytes;
     }
-    if (cfg->format == kSRGB16) {
-        // exact memo of the sRGB16 transfer function: one gather per sample instead of one powf
-        const size_t bytes = (size_t)65536 * sizeof(float);
-        CR(cudaMalloc(&h->eotf_lut, bytes));
-        k_build_srgb16_lut<<<65536 / 256, 256>>>(h->eotf_lut);
-        CR(cudaGetLastError());
-        CR(cudaDeviceSynchronize());
-        h->geo.eotf_lut = h->eotf_lut;
-        h->geo.lut_n = 65536;
-        h->geo.lut_shift = 0;
+    if (h->mixed) {
+        // the distorted side: same geometry, its own coefficients and memo table
+        size_t bytes = 0;
+        h->geo_dis = h->geo;
+        h->geo_dis.coef = make_coef(dis->format, dis->matrix, dis->full_range);
+        h->geo_dis.eotf_lut = nullptr;
+        h->geo_dis.lut_n = h->geo_dis.lut_shift = 0;
+        CR(build_side_lut(h->fmt[1], deep_dis, h->geo_dis, &h->eotf_lut_dis, &bytes));
         h->device_bytes += bytes;
     }
     for (uint32_t i = 0; i < h->ring; i++) {
@@ -669,6 +791,7 @@ int ssimu2_destroy(ssimu2_t* h)
     }
     cudaFree(h->scores_ring_d);
     cudaFree(h->eotf_lut);
+    cudaFree(h->eotf_lut_dis);
     delete h;
     return SSIMU2_OK;
 }
@@ -682,7 +805,7 @@ int ssimu2_mem_usage(const ssimu2_t* h, size_t* bytes)
 
 int ssimu2_submit(ssimu2_t* h, const ssimu2_frame* ref, const ssimu2_frame* dis, void* stream, uint64_t* ticket)
 {
-    if (!h || !frame_ok(h, ref) || !frame_ok(h, dis)) return SSIMU2_E_INVALID;
+    if (!h || !frame_ok(h, ref, 0) || !frame_ok(h, dis, 1)) return SSIMU2_E_INVALID;
     DeviceGuard guard(h->cfg.device);
     int r = prepare_cur(h);
     if (r) return r;
@@ -710,50 +833,24 @@ int ssimu2_submit_batch(ssimu2_t* h, uint32_t n, const ssimu2_frame* refs, const
 
 int ssimu2_submit_host(ssimu2_t* h, const ssimu2_frame* ref, const ssimu2_frame* dis, size_t frame_bytes, uint64_t* ticket)
 {
-    if (!h || !frame_ok(h, ref) || !frame_ok(h, dis) || frame_bytes == 0) return SSIMU2_E_INVALID;
-    const bool yuv = h->cfg.format == kNV12 || h->cfg.format == kP016;
-    if (yuv && (ref->plane[1] <= ref->plane[0] || dis->plane[1] <= dis->plane[0] ||
-                ref->plane[1] - ref->plane[0] >= frame_bytes || dis->plane[1] - dis->plane[0] >= frame_bytes))
-        return SSIMU2_E_INVALID;
-    DeviceGuard guard(h->cfg.device);
-    if (frame_bytes > h->staging_frame_bytes) {
-        // (re)allocate the staging rings; rare (first call), so a full drain is acceptable
-        int fr = ssimu2_flush(h);
-        if (fr) return fr;
-        for (uint32_t i = 0; i < h->ring; i++) {
-            int r = harvest(h, i);
-            if (r) return r;
-        }
-        size_t fb = (frame_bytes + 255) / 256 * 256;
-        for (auto& sl : h->slots) {
-            cudaFree(sl.staging);
-            sl.staging = nullptr;
-            if (cudaMalloc(&sl.staging, fb * 2 * h->batch) != cudaSuccess) { cudaGetLastError(); return SSIMU2_E_NOMEM; }
-        }
-        h->device_bytes += (fb - h->staging_frame_bytes) * 2 * h->batch * h->ring;
-        h->staging_frame_bytes = fb;
-    }
-    int r = prepare_cur(h);
-    if (r) return r;
-    Slot& sl = h->slots[h->cur];
-    uint8_t* da = sl.staging + (size_t)(2 * sl.count) * h->staging_frame_bytes;
-    uint8_t* db = da + h->staging_frame_bytes;
-    CU_TRY(cudaMemcpyAsync(da, (const void*)ref->plane[0], frame_bytes, cudaMemcpyHostToDevice, sl.stream));
-    CU_TRY(cudaMemcpyAsync(db, (const void*)dis->plane[0], frame_bytes, cudaMemcpyHostToDevice, sl.stream));
-    FramePair& fp = sl.in_h[sl.count];
-    fp.ref.p0 = da; fp.ref.p1 = yuv ? da + (ref->plane[1] - ref->plane[0]) : nullptr; fp.ref.pitch = ref->pitch; fp.ref.pad = 0;
-    fp.dis.p0 = db; fp.dis.p1 = yuv ? db + (dis->plane[1] - dis->plane[0]) : nullptr; fp.dis.pitch = dis->pitch; fp.dis.pad = 0;
-    if (ticket) *ticket = h->next_ticket;
-    return finish_pair(h);
+    return ssimu2_submit_host_batch(h, 1, ref, dis, frame_bytes, ticket);
 }
 
 int ssimu2_submit_host_batch(ssimu2_t* h, uint32_t n, const ssimu2_frame* refs, const ssimu2_frame* diss, size_t frame_bytes,
                              uint64_t* first_ticket)
 {
+    // one byte count for both frames: only meaningful when the two sides have the same bytes per pixel
+    if (h && in_bytes_per_px(h->fmt[0]) != in_bytes_per_px(h->fmt[1])) return SSIMU2_E_INVALID;
+    return ssimu2_submit_host_sized(h, n, refs, frame_bytes, diss, frame_bytes, first_ticket);
+}
+
+int ssimu2_submit_host_sized(ssimu2_t* h, uint32_t n, const ssimu2_frame* refs, size_t ref_bytes, const ssimu2_frame* diss,
+                             size_t dis_bytes, uint64_t* first_ticket)
+{
     if (!h || (n && (!refs || !diss))) return SSIMU2_E_INVALID;
     if (first_ticket) *first_ticket = h->next_ticket;
     for (uint32_t i = 0; i < n; i++) {
-        int r = ssimu2_submit_host(h, &refs[i], &diss[i], frame_bytes, nullptr);
+        int r = submit_host_pair(h, &refs[i], ref_bytes, &diss[i], dis_bytes);
         if (r) return r;
     }
     return SSIMU2_OK;

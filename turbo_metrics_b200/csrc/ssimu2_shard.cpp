@@ -25,7 +25,8 @@ constexpr uint64_t kShardResultCap = 1u << 16;   // global tickets kept in the r
 
 struct Job {
     ssimu2_frame ref, dis;
-    size_t frame_bytes;    // host frames: bytes to copy; 0 = device frames
+    size_t frame_bytes;    // host frames: bytes to copy (of the reference frame when dis_bytes != 0); 0 = device frames
+    size_t dis_bytes;      // host frames of ssimu2_shard_submit_host_sized: bytes of the distorted frame
     void* stream;          // device frames: producer stream on that device
     uint64_t global;       // global ticket
 };
@@ -49,6 +50,8 @@ struct Worker {
 
 struct ssimu2_shard {
     ssimu2_config cfg{};
+    ssimu2_source dis{};             // the distorted frames' description (has_dis: ssimu2_shard_create_mixed)
+    bool has_dis = false;
     uint32_t batch = 0;
     std::vector<Worker*> workers;
     uint64_t next_global = 0;
@@ -85,7 +88,7 @@ void worker_main(ssimu2_shard* s, Worker* w)
     {
         ssimu2_config c = s->cfg;
         c.device = w->device;
-        const int rc = ssimu2_create(&w->h, &c);
+        const int rc = ssimu2_create_mixed(&w->h, &c, s->has_dis ? &s->dis : nullptr);
         std::lock_guard<std::mutex> lk(w->mu);
         w->create_rc = rc;
         w->ready = true;
@@ -109,8 +112,9 @@ void worker_main(ssimu2_shard* s, Worker* w)
             w->global_of[w->submitted % w->global_of.size()] = j.global;
             w->submitted++;
             lk.unlock();
-            const int rc = j.frame_bytes ? ssimu2_submit_host(w->h, &j.ref, &j.dis, j.frame_bytes, nullptr)
-                                         : ssimu2_submit(w->h, &j.ref, &j.dis, j.stream, nullptr);
+            const int rc = j.dis_bytes     ? ssimu2_submit_host_sized(w->h, 1, &j.ref, j.frame_bytes, &j.dis, j.dis_bytes, nullptr)
+                           : j.frame_bytes ? ssimu2_submit_host(w->h, &j.ref, &j.dis, j.frame_bytes, nullptr)
+                                           : ssimu2_submit(w->h, &j.ref, &j.dis, j.stream, nullptr);
             if (rc) fail(s, rc);
             lk.lock();
             continue;
@@ -144,7 +148,7 @@ inline void route(const ssimu2_shard* s, uint64_t g, uint32_t* wi, uint64_t* loc
 }
 
 int submit_common(ssimu2_shard* s, uint32_t n, const ssimu2_frame* refs, const ssimu2_frame* diss, size_t frame_bytes,
-                  void* const* streams, uint64_t* first_ticket)
+                  size_t dis_bytes, void* const* streams, uint64_t* first_ticket)
 {
     if (!s || (n && (!refs || !diss))) return SSIMU2_E_INVALID;
     if (int e = s->error.load()) return e;
@@ -165,7 +169,7 @@ int submit_common(ssimu2_shard* s, uint32_t n, const ssimu2_frame* refs, const s
         {
             std::lock_guard<std::mutex> lk(w->mu);
             for (uint32_t k = 0; k < m; k++)
-                w->queue.push_back(Job{refs[i + k], diss[i + k], frame_bytes, streams ? streams[wi] : nullptr, s->next_global + k});
+                w->queue.push_back(Job{refs[i + k], diss[i + k], frame_bytes, dis_bytes, streams ? streams[wi] : nullptr, s->next_global + k});
             w->cv.notify_one();
         }
         s->next_global += m;
@@ -180,11 +184,21 @@ extern "C" {
 
 int ssimu2_shard_create(ssimu2_shard_t** out, const ssimu2_config* cfg, const int32_t* devices, uint32_t n_devices)
 {
+    return ssimu2_shard_create_mixed(out, cfg, nullptr, devices, n_devices);
+}
+
+int ssimu2_shard_create_mixed(ssimu2_shard_t** out, const ssimu2_config* cfg, const ssimu2_source* dis, const int32_t* devices,
+                              uint32_t n_devices)
+{
     if (!out || !cfg || !devices || n_devices == 0 || n_devices > 64) return SSIMU2_E_INVALID;
     *out = nullptr;
     ssimu2_shard* s = new (std::nothrow) ssimu2_shard();
     if (!s) return SSIMU2_E_NOMEM;
     s->cfg = *cfg;
+    if (dis) {
+        s->dis = *dis;
+        s->has_dis = true;
+    }
     s->batch = cfg->batch ? cfg->batch : 8;
     if (s->batch > 1024) s->batch = 1024;
     s->cfg.batch = s->batch;
@@ -237,13 +251,20 @@ int ssimu2_shard_submit_host(ssimu2_shard_t* s, uint32_t n, const ssimu2_frame* 
                              uint64_t* first_ticket)
 {
     if (frame_bytes == 0) return SSIMU2_E_INVALID;
-    return submit_common(s, n, refs, diss, frame_bytes, nullptr, first_ticket);
+    return submit_common(s, n, refs, diss, frame_bytes, 0, nullptr, first_ticket);
+}
+
+int ssimu2_shard_submit_host_sized(ssimu2_shard_t* s, uint32_t n, const ssimu2_frame* refs, size_t ref_bytes, const ssimu2_frame* diss,
+                                   size_t dis_bytes, uint64_t* first_ticket)
+{
+    if (ref_bytes == 0 || dis_bytes == 0) return SSIMU2_E_INVALID;
+    return submit_common(s, n, refs, diss, ref_bytes, dis_bytes, nullptr, first_ticket);
 }
 
 int ssimu2_shard_submit_device(ssimu2_shard_t* s, uint32_t n, const ssimu2_frame* refs, const ssimu2_frame* diss, void* const* streams,
                                uint64_t* first_ticket)
 {
-    return submit_common(s, n, refs, diss, 0, streams, first_ticket);
+    return submit_common(s, n, refs, diss, 0, 0, streams, first_ticket);
 }
 
 int ssimu2_shard_device_of(const ssimu2_shard_t* s, uint64_t ticket, int32_t* device)

@@ -19,7 +19,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import Config, Frame, Info, check
+from ._lib import Config, Frame, Info, Source, check
 
 
 class PixelFormat(IntEnum):
@@ -86,19 +86,51 @@ def make_config(width, height, fmt, matrix=ColorMatrix.BT709, full_range=False, 
     return cfg
 
 
+def make_source(cfg: Config, dis_fmt=None, dis_matrix=None, dis_full_range=None, dis_p016_deep=None) -> Optional[Source]:
+    """ssimu2_source of the distorted frames for a handle whose reference frames `cfg` describes, or None when no dis_*
+    argument is given.  A dis_* argument left at None takes the reference's value; the deep flag is the reference's when the
+    distorted frames are P016 too."""
+    if dis_fmt is None and dis_matrix is None and dis_full_range is None and dis_p016_deep is None:
+        return None
+    src = Source()
+    src.format = int(cfg.format if dis_fmt is None else dis_fmt)
+    src.matrix = int(cfg.matrix if dis_matrix is None else dis_matrix)
+    src.full_range = int(cfg.full_range if dis_full_range is None else dis_full_range)
+    if dis_p016_deep is None:
+        dis_p016_deep = bool(cfg.flags & _lib.FLAG_P016_DEEP) and src.format == PixelFormat.P016
+    src.flags = _lib.FLAG_P016_DEEP if dis_p016_deep else 0
+    return src
+
+
+def is_mixed(cfg: Config, src: Optional[Source]) -> bool:
+    """Whether ssimu2_create_mixed(cfg, src) makes a mixed handle: the sides differ in format or deep flag, or (NV12 / P016) in
+    matrix or range.  Otherwise the handle is an ordinary one."""
+    if src is None:
+        return False
+    deep = _lib.FLAG_P016_DEEP
+    yuv = cfg.format in (PixelFormat.NV12, PixelFormat.P016)
+    return not (src.format == cfg.format and (src.flags & deep) == (cfg.flags & deep) and
+                (not yuv or (src.matrix == cfg.matrix and bool(src.full_range) == bool(cfg.full_range))))
+
+
 class Ssimulacra2:
     """`Ssimulacra2::new` (lib.rs:48-107): an instance is valid for one width x height x format."""
 
     def __init__(self, width: int, height: int, fmt: PixelFormat = PixelFormat.LINEARF32,
                  matrix: ColorMatrix = ColorMatrix.BT709, full_range: bool = False, device: int = 0,
                  batch: int = 0, ring: int = 0, pipeline: Optional[str] = None, score_only: bool = False,
-                 input_group: int = 0, timing: bool = True, p016_deep: bool = False):
+                 input_group: int = 0, timing: bool = True, p016_deep: bool = False, dis_fmt: Optional[PixelFormat] = None,
+                 dis_matrix: Optional[ColorMatrix] = None, dis_full_range: Optional[bool] = None,
+                 dis_p016_deep: Optional[bool] = None):
         """pipeline: None / "hv" = the product pipeline (front-end, fused H+V kernel, finalize); "split" = development
         pipeline with the H-pass planes in HBM (debug_read(what=1)).
         score_only: SSIMU2_FLAG_SCORE_ONLY -- skip the work whose weights are zero (scores identical, no norms).
         input_group: pairs per front-end launch (0 = whole batch): input frames are consumed sooner, see wait_input().
         p016_deep: SSIMU2_FLAG_P016_DEEP -- P016 samples with more than 10 significant bits (12-bit sources): same results,
-        a front-end without the 10-bit memo tables."""
+        a front-end without the 10-bit memo tables (of the reference frames when the distorted frames are described apart).
+        dis_fmt, dis_matrix, dis_full_range, dis_p016_deep: the distorted frames' own description (None = as the reference);
+        any of them set creates the handle with ssimu2_create_mixed.  Host frames of a mixed handle are copied with each
+        side's own `nbytes`."""
         self._h = C.c_void_p()
         if pipeline not in (None, "hv", "split"):
             raise ValueError(f"unknown pipeline {pipeline!r}")
@@ -106,8 +138,14 @@ class Ssimulacra2:
                 (_lib.FLAG_P016_DEEP if p016_deep else 0)
         cfg = make_config(width, height, fmt, matrix, full_range, device, batch, ring,
                           _lib.PIPELINE_SPLIT if pipeline == "split" else _lib.PIPELINE_DEFAULT, flags, input_group)
-        check(_lib.lib().ssimu2_create(C.byref(self._h), C.byref(cfg)), "ssimu2_create")
+        src = make_source(cfg, dis_fmt, dis_matrix, dis_full_range, dis_p016_deep)
+        if src is None:
+            check(_lib.lib().ssimu2_create(C.byref(self._h), C.byref(cfg)), "ssimu2_create")
+        else:
+            check(_lib.lib().ssimu2_create_mixed(C.byref(self._h), C.byref(cfg), C.byref(src)), "ssimu2_create_mixed")
         self.width, self.height, self.format = width, height, PixelFormat(fmt)
+        self.dis_format = self.format if src is None else PixelFormat(src.format)
+        self.mixed = is_mixed(cfg, src)
         self._keep = {}
         self._last = None
 
@@ -179,21 +217,32 @@ class Ssimulacra2:
         host memory; the library stages them on the device."""
         t = C.c_uint64()
         a, b = ref.c(), dis.c()
-        assert ref.nbytes and ref.nbytes == dis.nbytes
-        check(_lib.lib().ssimu2_submit_host(self._h, C.byref(a), C.byref(b), ref.nbytes, C.byref(t)),
-              "ssimu2_submit_host")
+        if self.mixed:
+            assert ref.nbytes and dis.nbytes
+            check(_lib.lib().ssimu2_submit_host_sized(self._h, 1, C.byref(a), ref.nbytes, C.byref(b), dis.nbytes, C.byref(t)),
+                  "ssimu2_submit_host_sized")
+        else:
+            assert ref.nbytes and ref.nbytes == dis.nbytes
+            check(_lib.lib().ssimu2_submit_host(self._h, C.byref(a), C.byref(b), ref.nbytes, C.byref(t)),
+                  "ssimu2_submit_host")
         self._keep[t.value] = (ref, dis)
         self._last = t.value
         return t.value
 
     def compute_from_cpu_batch(self, refs: Sequence[DeviceFrame], diss: Sequence[DeviceFrame]) -> range:
-        """n host pairs in one call (`ssimu2_submit_host_batch`)."""
+        """n host pairs in one call (`ssimu2_submit_host_batch`; `ssimu2_submit_host_sized` on a mixed handle)."""
         n = len(refs)
-        assert n == len(diss) and n > 0 and all(f.nbytes == refs[0].nbytes for f in list(refs) + list(diss))
+        assert n == len(diss) and n > 0
         A = (Frame * n)(*[f.c() for f in refs])
         B = (Frame * n)(*[f.c() for f in diss])
         t = C.c_uint64()
-        check(_lib.lib().ssimu2_submit_host_batch(self._h, n, A, B, refs[0].nbytes, C.byref(t)), "ssimu2_submit_host_batch")
+        if self.mixed:
+            assert all(f.nbytes == refs[0].nbytes for f in refs) and all(f.nbytes == diss[0].nbytes for f in diss)
+            check(_lib.lib().ssimu2_submit_host_sized(self._h, n, A, refs[0].nbytes, B, diss[0].nbytes, C.byref(t)),
+                  "ssimu2_submit_host_sized")
+        else:
+            assert all(f.nbytes == refs[0].nbytes for f in list(refs) + list(diss))
+            check(_lib.lib().ssimu2_submit_host_batch(self._h, n, A, B, refs[0].nbytes, C.byref(t)), "ssimu2_submit_host_batch")
         for i in range(n):
             self._keep[t.value + i] = (refs[i], diss[i])
         self._last = t.value + n - 1
@@ -292,12 +341,21 @@ class ShardedSsimulacra2:
     (ssimulacra2-cuda/README.md:26-27), the reference's single-GPU frame loop is turbo-metrics/src/lib.rs:362-433."""
 
     def __init__(self, width: int, height: int, fmt: PixelFormat, devices: Sequence[int], matrix: ColorMatrix = ColorMatrix.BT709,
-                 full_range: bool = False, batch: int = 0, ring: int = 0, score_only: bool = False):
+                 full_range: bool = False, batch: int = 0, ring: int = 0, score_only: bool = False,
+                 dis_fmt: Optional[PixelFormat] = None, dis_matrix: Optional[ColorMatrix] = None,
+                 dis_full_range: Optional[bool] = None, dis_p016_deep: Optional[bool] = None):
+        """dis_*: the distorted frames' own description, as for `Ssimulacra2` (every worker's handle is ssimu2_create_mixed)."""
         self._s = C.c_void_p()
         flags = _lib.FLAG_SCORE_ONLY if score_only else 0
         cfg = make_config(width, height, fmt, matrix, full_range, 0, batch, ring, _lib.PIPELINE_DEFAULT, flags, 0)
         devs = (C.c_int32 * len(devices))(*devices)
-        check(_lib.lib().ssimu2_shard_create(C.byref(self._s), C.byref(cfg), devs, len(devices)), "ssimu2_shard_create")
+        src = make_source(cfg, dis_fmt, dis_matrix, dis_full_range, dis_p016_deep)
+        if src is None:
+            check(_lib.lib().ssimu2_shard_create(C.byref(self._s), C.byref(cfg), devs, len(devices)), "ssimu2_shard_create")
+        else:
+            check(_lib.lib().ssimu2_shard_create_mixed(C.byref(self._s), C.byref(cfg), C.byref(src), devs, len(devices)),
+                  "ssimu2_shard_create_mixed")
+        self.mixed = is_mixed(cfg, src)
         self.devices = list(devices)
         self._keep = []
         self._done_upto = 0
@@ -331,7 +389,11 @@ class ShardedSsimulacra2:
         A = (Frame * n)(*[f.c() for f in refs])
         B = (Frame * n)(*[f.c() for f in diss])
         t = C.c_uint64()
-        check(_lib.lib().ssimu2_shard_submit_host(self._s, n, A, B, refs[0].nbytes, C.byref(t)), "ssimu2_shard_submit_host")
+        if self.mixed:
+            check(_lib.lib().ssimu2_shard_submit_host_sized(self._s, n, A, refs[0].nbytes, B, diss[0].nbytes, C.byref(t)),
+                  "ssimu2_shard_submit_host_sized")
+        else:
+            check(_lib.lib().ssimu2_shard_submit_host(self._s, n, A, B, refs[0].nbytes, C.byref(t)), "ssimu2_shard_submit_host")
         self._keep.append((t.value + n, refs, diss))
         return range(t.value, t.value + n)
 
