@@ -85,9 +85,18 @@ typedef enum {
 typedef enum { SSIMU2_MATRIX_BT709 = 0, SSIMU2_MATRIX_BT601_525 = 1, SSIMU2_MATRIX_BT601_625 = 2 } ssimu2_matrix;
 
 /* One device frame.  YUV 4:2:0: plane[0] = Y, plane[1] = interleaved CbCr
- * (NVDEC: plane[1] = plane[0] + pitch * coded_height, cudarse-video/src/dec.rs:299-366),
- * both with the same pitch.  Packed RGB formats use plane[0] only.  pitch is in bytes and must hold one row
- * (width x 1 / 2 bytes for NV12 / P016, width x 3 / 6 / 12 bytes for the packed formats): SSIMU2_E_INVALID otherwise. */
+ * (NVDEC: plane[1] = plane[0] + pitch * coded_height, cudarse-video/src/dec.rs:299-366, but any placement works: a separate
+ * allocation, chroma before luma, coded_height == height), both with the same pitch.  Packed RGB formats use plane[0] only.
+ * Layout rule (SSIMU2_E_INVALID otherwise, ABI 2.2):
+ *   - pitch is in bytes and holds one row: width x 3 / 6 / 12 bytes for sRGB8 / sRGB16 / the f32 formats; for NV12 / P016
+ *     width luma samples and 2 x ceil(width / 2) chroma samples (1 / 2 bytes each);
+ *   - everything is aligned to one sample (1 byte: NV12, sRGB8; 2: P016, sRGB16; 4: sRGB f32, linear f32): for device frames
+ *     plane[0], plane[1] and pitch; for host frames pitch and plane[1] - plane[0] (host frames are staged to aligned memory);
+ *   - host frames: the byte count copied from plane[0] covers (height - 1) x pitch + the row bytes and, for YUV, the end of the
+ *     last chroma row, (plane[1] - plane[0]) + (ceil(height / 2) - 1) x pitch + the chroma row bytes.
+ * Rows may be padded and may lie more than 4 GiB past plane[0].  The batch entry points (ssimu2_submit_batch,
+ * ssimu2_submit_host_batch / _sized, ssimu2_shard_submit_*) check every pair before queueing any: on SSIMU2_E_INVALID nothing of
+ * the call was accepted. */
 typedef struct {
     uint64_t plane[2];
     uint32_t pitch;

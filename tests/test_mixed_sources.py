@@ -27,10 +27,11 @@ def _src(**kw):
 
 
 # ------------------------------------------------------------------------------------------ CPU
-def test_source_layout_and_version():
+def test_source_layout_and_minimum_version():
+    """ssimu2_source is 32 bytes and the library has the mixed-source calls of ABI 2.1 (later minor versions only add)."""
     from turbo_metrics_b200 import _lib
     assert C.sizeof(_lib.Source) == 32
-    assert _lib.lib().ssimu2_version() == (2 << 16) | 1
+    assert _lib.lib().ssimu2_version() >= (2 << 16) | 1
 
 
 def test_create_mixed_rejects_bad_sources_without_a_device():

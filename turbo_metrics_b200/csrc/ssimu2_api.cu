@@ -12,6 +12,7 @@
 // There is no CPU fallback: without a usable CUDA device every call fails.
 #include "../../include/ssimu2_b200.h"
 #include "../../include/ssimu2_b200_debug.h"
+#include "frame_layout.h"
 #include "ssimu2_kernels.cuh"
 
 #include <cstdio>
@@ -499,16 +500,11 @@ static int finish_pair(ssimu2_handle* h)
 
 static bool is_yuv(int fmt) { return fmt == kNV12 || fmt == kP016; }
 
-// side 0: a reference frame, 1: a distorted frame (each side is checked against its own format)
-static bool frame_ok(const ssimu2_handle* h, const ssimu2_frame* f, int side)
+// side 0: a reference frame, 1: a distorted frame (each side is checked against its own format); host frames with the byte
+// count copied from plane[0]
+static bool frame_ok(const ssimu2_handle* h, const ssimu2_frame* f, int side, bool host = false, size_t bytes = 0)
 {
-    const int fmt = h->fmt[side];
-    if (!f || !f->plane[0] || f->pitch == 0) return false;
-    if (is_yuv(fmt) && !f->plane[1]) return false;
-    // a row must fit in the pitch (rows that overlap would be read as garbage, and past the end of the last one)
-    static const uint32_t bytes_per_px[] = {1, 2, 3, 6, 12, 12};   // NV12 / P016: per luma sample; packed RGB: per pixel
-    if ((uint64_t)f->pitch < (uint64_t)h->cfg.width * bytes_per_px[fmt]) return false;
-    return true;
+    return frame_layout_ok(h->fmt[side], h->cfg.width, h->cfg.height, f, host, bytes);
 }
 
 // locate a ticket: 0 = results on host, 1 = in a launched slot, 2 = in the slot being filled
@@ -557,10 +553,8 @@ static int note_dependency(Slot& sl, void* stream)
 // one host pair: copy each frame (its own byte count) to the slot's staging ring and record the pair
 static int submit_host_pair(ssimu2_handle* h, const ssimu2_frame* ref, size_t ref_bytes, const ssimu2_frame* dis, size_t dis_bytes)
 {
-    if (!frame_ok(h, ref, 0) || !frame_ok(h, dis, 1) || ref_bytes == 0 || dis_bytes == 0) return SSIMU2_E_INVALID;
+    if (!frame_ok(h, ref, 0, true, ref_bytes) || !frame_ok(h, dis, 1, true, dis_bytes)) return SSIMU2_E_INVALID;
     const bool yuv_ref = is_yuv(h->fmt[0]), yuv_dis = is_yuv(h->fmt[1]);
-    if (yuv_ref && (ref->plane[1] <= ref->plane[0] || ref->plane[1] - ref->plane[0] >= ref_bytes)) return SSIMU2_E_INVALID;
-    if (yuv_dis && (dis->plane[1] <= dis->plane[0] || dis->plane[1] - dis->plane[0] >= dis_bytes)) return SSIMU2_E_INVALID;
     DeviceGuard guard(h->cfg.device);
     const size_t frame_bytes = ref_bytes > dis_bytes ? ref_bytes : dis_bytes;
     if (frame_bytes > h->staging_frame_bytes) {
@@ -597,7 +591,7 @@ static int submit_host_pair(ssimu2_handle* h, const ssimu2_frame* ref, size_t re
 
 extern "C" {
 
-uint32_t ssimu2_version(void) { return (2u << 16) | 1u; }
+uint32_t ssimu2_version(void) { return (2u << 16) | 2u; }
 
 const char* ssimu2_strerror(int status)
 {
@@ -823,6 +817,9 @@ int ssimu2_submit_batch(ssimu2_t* h, uint32_t n, const ssimu2_frame* refs, const
                         uint64_t* first_ticket)
 {
     if (!h || (n && (!refs || !diss))) return SSIMU2_E_INVALID;
+    // all or nothing: every pair is checked before the first one is queued
+    for (uint32_t i = 0; i < n; i++)
+        if (!frame_ok(h, &refs[i], 0) || !frame_ok(h, &diss[i], 1)) return SSIMU2_E_INVALID;
     if (first_ticket) *first_ticket = h->next_ticket;
     for (uint32_t i = 0; i < n; i++) {
         int r = ssimu2_submit(h, &refs[i], &diss[i], stream, nullptr);
@@ -848,6 +845,8 @@ int ssimu2_submit_host_sized(ssimu2_t* h, uint32_t n, const ssimu2_frame* refs, 
                              size_t dis_bytes, uint64_t* first_ticket)
 {
     if (!h || (n && (!refs || !diss))) return SSIMU2_E_INVALID;
+    for (uint32_t i = 0; i < n; i++)
+        if (!frame_ok(h, &refs[i], 0, true, ref_bytes) || !frame_ok(h, &diss[i], 1, true, dis_bytes)) return SSIMU2_E_INVALID;
     if (first_ticket) *first_ticket = h->next_ticket;
     for (uint32_t i = 0; i < n; i++) {
         int r = submit_host_pair(h, &refs[i], ref_bytes, &diss[i], dis_bytes);

@@ -9,6 +9,7 @@
 // (g / batch) % n, so whole launch groups stay on one GPU and consecutive groups rotate over the GPUs.
 // Only the public C API of the scorer is used here: no CUDA calls, no torch, no NCCL.
 #include "../../include/ssimu2_b200.h"
+#include "frame_layout.h"
 
 #include <atomic>
 #include <condition_variable>
@@ -152,6 +153,13 @@ int submit_common(ssimu2_shard* s, uint32_t n, const ssimu2_frame* refs, const s
 {
     if (!s || (n && (!refs || !diss))) return SSIMU2_E_INVALID;
     if (int e = s->error.load()) return e;
+    // every frame is checked here, before any is queued: a frame the worker rejected later would fail the whole shard
+    const bool host = frame_bytes != 0;
+    const int ref_fmt = s->cfg.format, dis_fmt = s->has_dis ? s->dis.format : s->cfg.format;
+    for (uint32_t i = 0; i < n; i++)
+        if (!frame_layout_ok(ref_fmt, s->cfg.width, s->cfg.height, &refs[i], host, frame_bytes) ||
+            !frame_layout_ok(dis_fmt, s->cfg.width, s->cfg.height, &diss[i], host, dis_bytes ? dis_bytes : frame_bytes))
+            return SSIMU2_E_INVALID;
     if (first_ticket) *first_ticket = s->next_global;
     uint32_t i = 0;
     while (i < n) {

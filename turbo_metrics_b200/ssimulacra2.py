@@ -66,15 +66,23 @@ class DeviceFrame:
 
     @staticmethod
     def packed(img, pitch: Optional[int] = None) -> "DeviceFrame":
-        """Packed RGB image (H, W, 3) of u8 / u16 / f32: NPP `Image<_, C<3>>` layout."""
-        base = img.data_ptr() if hasattr(img, "data_ptr") else img.ctypes.data
+        """Packed RGB image (H, W, 3) of u8 / u16 / f32, or its rows as (H, 3 * W): NPP `Image<_, C<3>>` layout.  Rows may be
+        padded (a view such as img[:, :w] of a wider image), but the samples of a row must be packed: ValueError otherwise.
+        `nbytes` is the span from the first sample to the last, what compute_from_cpu copies."""
+        if hasattr(img, "data_ptr"):
+            base, esize = img.data_ptr(), img.element_size()
+            strides = tuple(s * esize for s in img.stride())
+        else:
+            base, esize, strides = img.ctypes.data, img.itemsize, tuple(img.strides)
+        shape = tuple(img.shape)
+        packed = (len(shape) == 3 and shape[2] == 3 and strides[1:] == (3 * esize, esize)) or \
+                 (len(shape) == 2 and strides[1] == esize)
+        if not packed:
+            raise ValueError(f"not a packed RGB image: shape {shape}, byte strides {strides}")
         if pitch is None:
-            if hasattr(img, "stride"):
-                pitch = img.stride(0) * img.element_size()
-            else:
-                pitch = img.strides[0]
-        nbytes = img.numel() * img.element_size() if hasattr(img, "numel") else img.nbytes
-        return DeviceFrame(base, 0, pitch, img, nbytes)
+            pitch = strides[0]
+        row = int(np.prod(shape[1:])) * esize
+        return DeviceFrame(base, 0, pitch, img, (shape[0] - 1) * pitch + row)
 
 
 def make_config(width, height, fmt, matrix=ColorMatrix.BT709, full_range=False, device=0, batch=0, ring=0,
