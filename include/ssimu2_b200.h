@@ -78,22 +78,35 @@ typedef enum {
     SSIMU2_FMT_SRGB8 = 2,     /* Npp8 : packed RGB u8, sRGB transfer (256-entry table) */
     SSIMU2_FMT_SRGB16 = 3,    /* Npp16: packed RGB u16, sRGB transfer (analytic) */
     SSIMU2_FMT_SRGBF32 = 4,   /* Npp32: packed RGB f32 in [0,1], sRGB transfer (analytic) */
-    SSIMU2_FMT_LINEARF32 = 5  /* packed linear RGB f32: the input of Ssimulacra2::new itself */
+    SSIMU2_FMT_LINEARF32 = 5, /* packed linear RGB f32: the input of Ssimulacra2::new itself */
+    /* ABI 2.3: NVDEC's 4:2:2 and 4:4:4 surfaces (cudaVideoSurfaceFormat_NV16 / _P216 / _YUV444 / _YUV444_16Bit).  Chroma is
+     * sited nearest-neighbour, like the 4:2:0 formats: pixel (x, y) takes chroma (x >> 1, y) in 4:2:2, (x, y) in 4:4:4. */
+    SSIMU2_FMT_NV16 = 8,      /* u8 Y plane + interleaved u8 CbCr plane of full height, 4:2:2 */
+    SSIMU2_FMT_P216 = 9,      /* u16 MSB-aligned Y + interleaved CbCr of full height, 4:2:2 */
+    SSIMU2_FMT_YUV444 = 10,   /* u8 Y, Cb and Cr planes, 4:4:4 */
+    SSIMU2_FMT_YUV444P16 = 11 /* u16 MSB-aligned Y, Cb and Cr planes, 4:4:4 */
 } ssimu2_format;
 
 /* cuda-colorspace/src/lib.rs:8-13 `ColorMatrix` (only used by the YUV formats). */
 typedef enum { SSIMU2_MATRIX_BT709 = 0, SSIMU2_MATRIX_BT601_525 = 1, SSIMU2_MATRIX_BT601_625 = 2 } ssimu2_matrix;
 
-/* One device frame.  YUV 4:2:0: plane[0] = Y, plane[1] = interleaved CbCr
+/* One device frame.  YUV 4:2:0: plane[0] = Y, plane[1] = interleaved CbCr, ceil(height / 2) rows
  * (NVDEC: plane[1] = plane[0] + pitch * coded_height, cudarse-video/src/dec.rs:299-366, but any placement works: a separate
- * allocation, chroma before luma, coded_height == height), both with the same pitch.  Packed RGB formats use plane[0] only.
- * Layout rule (SSIMU2_E_INVALID otherwise, ABI 2.2):
- *   - pitch is in bytes and holds one row: width x 3 / 6 / 12 bytes for sRGB8 / sRGB16 / the f32 formats; for NV12 / P016
- *     width luma samples and 2 x ceil(width / 2) chroma samples (1 / 2 bytes each);
- *   - everything is aligned to one sample (1 byte: NV12, sRGB8; 2: P016, sRGB16; 4: sRGB f32, linear f32): for device frames
- *     plane[0], plane[1] and pitch; for host frames pitch and plane[1] - plane[0] (host frames are staged to aligned memory);
+ * allocation, chroma before luma, coded_height == height), both with the same pitch.  YUV 4:2:2 (NV16, P216): the same with
+ * `height` rows of interleaved CbCr.  YUV 4:4:4 (YUV444, YUV444P16): plane[1] = Cb, and the Cr plane lies at
+ * plane[1] + (plane[1] - plane[0]), all three with the same pitch -- NVDEC's layout (planes pitch x coded_height apart) and that of
+ * a contiguous (3, H, pitch) array; ssimu2_frame has no third address.  Packed RGB formats use plane[0] only.
+ * Layout rule (SSIMU2_E_INVALID otherwise, ABI 2.2; 4:2:2 and 4:4:4 since 2.3):
+ *   - pitch is in bytes and holds one row: width x 3 / 6 / 12 bytes for sRGB8 / sRGB16 / the f32 formats; for NV12 / P016 /
+ *     NV16 / P216 width luma samples and 2 x ceil(width / 2) chroma samples, for YUV444 / YUV444P16 width samples (1 / 2 bytes
+ *     each);
+ *   - everything is aligned to one sample (1 byte: NV12, NV16, YUV444, sRGB8; 2: P016, P216, YUV444P16, sRGB16; 4: sRGB f32,
+ *     linear f32): for device frames plane[0], plane[1] and pitch (4:4:4: the Cr address must not wrap around the address space);
+ *     for host frames pitch and plane[1] - plane[0] (host frames are staged to aligned memory);
  *   - host frames: the byte count copied from plane[0] covers (height - 1) x pitch + the row bytes and, for YUV, the end of the
- *     last chroma row, (plane[1] - plane[0]) + (ceil(height / 2) - 1) x pitch + the chroma row bytes.
+ *     last chroma row: (plane[1] - plane[0]) + (ceil(height / 2) - 1) x pitch + the chroma row bytes for 4:2:0,
+ *     (plane[1] - plane[0]) + (height - 1) x pitch + the chroma row bytes for 4:2:2, 2 x (plane[1] - plane[0]) + (height - 1) x
+ *     pitch + the row bytes for 4:4:4 (the last Cr row).
  * Rows may be padded and may lie more than 4 GiB past plane[0].  The batch entry points (ssimu2_submit_batch,
  * ssimu2_submit_host_batch / _sized, ssimu2_shard_submit_*) check every pair before queueing any: on SSIMU2_E_INVALID nothing of
  * the call was accepted. */
@@ -114,8 +127,8 @@ typedef enum {
                                      by 0.0, ssimulacra2-cuda/src/lib.rs:586-603).  Scores are bit-identical to the full mode;    \
                                      ssimu2_get_norms returns SSIMU2_E_UNSUPPORTED. */
 #define SSIMU2_FLAG_NO_TIMING 2u  /* do not record the per-kernel timing events (ssimu2_b200_debug.h) */
-#define SSIMU2_FLAG_P016_DEEP 4u  /* SSIMU2_FMT_P016 only: the samples carry more than 10 significant bits (12-bit sources, e.g. HEVC \
-                                     Main12 through NVDEC).  Results never depend on this flag; it selects a front-end that      \
+#define SSIMU2_FLAG_P016_DEEP 4u  /* SSIMU2_FMT_P016, _P216 and _YUV444P16 only: the samples carry more than 10 significant bits \
+                                     (12-bit sources, e.g. HEVC Main12 / Main 4:4:4 12 through NVDEC).  Results never depend on this flag; it selects a front-end that      \
                                      evaluates all three transfer functions instead of the exact 10-bit memo tables, which such  \
                                      content cannot use (without the flag it is scored correctly, at a third of the speed). */
 
@@ -139,7 +152,7 @@ typedef struct {
     int32_t format;       /* ssimu2_format of the distorted frames */
     int32_t matrix;       /* ssimu2_matrix (YUV formats) */
     int32_t full_range;   /* 0 = limited, 1 = full */
-    uint32_t flags;       /* SSIMU2_FLAG_P016_DEEP only, and only with format == SSIMU2_FMT_P016 */
+    uint32_t flags;       /* SSIMU2_FLAG_P016_DEEP only, and only with a 16-bit YUV format (P016, P216, YUV444P16) */
     uint32_t reserved[4]; /* must be 0 */
 } ssimu2_source;
 
@@ -147,9 +160,9 @@ typedef struct {
 int ssimu2_create(ssimu2_t **out, const ssimu2_config *cfg);
 /* A handle whose distorted frames have their own pixel format / matrix / range.  cfg describes the reference frames (its
  * SSIMU2_FLAG_P016_DEEP applies to the reference side only); dis == NULL: exactly ssimu2_create.  `dis` is checked before any
- * device call: a bad format or matrix, a flag other than SSIMU2_FLAG_P016_DEEP, or that flag with a format other than P016 is
- * SSIMU2_E_UNSUPPORTED; non-zero reserved fields are SSIMU2_E_INVALID.  When the two sides are the same effective description
- * (same format and deep flag; for NV12 / P016 also the same matrix and range) the result is an ordinary handle: one
+ * device call: a bad format or matrix, a flag other than SSIMU2_FLAG_P016_DEEP, or that flag with a format other than P016 / P216
+ * / YUV444P16 is SSIMU2_E_UNSUPPORTED; non-zero reserved fields are SSIMU2_E_INVALID.  When the two sides are the same effective description
+ * (same format and deep flag; for the YUV formats also the same matrix and range) the result is an ordinary handle: one
  * front-end launch per input group and the same bits.  Otherwise the front-end runs once per side on the slot's stream, and
  * the frames of each side are checked against that side's format (ssimu2_frame pitch rule). */
 int ssimu2_create_mixed(ssimu2_t **out, const ssimu2_config *cfg, const ssimu2_source *dis);

@@ -91,7 +91,7 @@ struct ssimu2_handle {
     // side, the distorted side with geo_dis (geo with that side's coefficients and memo table)
     bool mixed = false;
     int fmt[2] = {0, 0};              // ssimu2_format of the reference / distorted frames
-    int fe_fmt[2] = {0, 0};           // their front-end formats (kP016A: P016 with SSIMU2_FLAG_P016_DEEP)
+    int fe_fmt[2] = {0, 0};           // their front-end formats (kP016A / kP216A / kYUV444P16A: with SSIMU2_FLAG_P016_DEEP)
     Geo geo_dis{};
     float* eotf_lut_dis = nullptr;
     uint32_t batch = 0, ring = 0, input_group = 0;
@@ -140,8 +140,8 @@ static void luma_constants(int matrix, float& kr, float& kb)
 static YuvCoef make_coef(int fmt, int matrix, int full_range)
 {
     YuvCoef c{};
-    if (fmt != kNV12 && fmt != kP016) return c;
-    int bits = fmt == kNV12 ? 8 : 16;
+    if (!format_is_yuv(fmt)) return c;
+    int bits = format_is_yuv16(fmt) ? 16 : 8;
     float kr, kb;
     luma_constants(matrix, kr, kb);
     uint32_t lmin, lrange, crange;
@@ -163,11 +163,18 @@ static YuvCoef make_coef(int fmt, int matrix, int full_range)
     return c;
 }
 
+// the front-end format of a 16-bit YUV side with SSIMU2_FLAG_P016_DEEP
+static int deep_fe_fmt(int fmt) { return fmt == kP016 ? kP016A : fmt == kP216 ? kP216A : kYUV444P16A; }
+
 static int in_bytes_per_px(int fmt)
 {
     switch (fmt) {
     case kNV12: return 3;       // 1.5 B x 2 images
     case kP016: return 6;
+    case kNV16: return 4;       // 2 B x 2 images
+    case kP216: return 8;
+    case kYUV444: return 6;
+    case kYUV444P16: return 12;
     case kSRGB8: return 6;
     case kSRGB16: return 12;
     default: return 24;
@@ -220,12 +227,14 @@ static void build_geo(ssimu2_handle* h)
 }
 
 // Exact memo of one side's transfer function (Geo::eotf_lut), built by the device code it replaces: the R / B tables of
-// 10-bit P016 and NV12, the sRGB16 table.  The other formats (and deep P016) have none.
+// 10-bit P016 and NV12 (also those of P216 / YUV444P16 and NV16 / YUV444: the tables are indexed per pixel by (Cr, Y) and
+// (Cb, Y), whatever the subsampling), the sRGB16 table.  The other formats (and the deep 16-bit YUV sides) have none.
 static cudaError_t build_side_lut(int fmt, bool deep, Geo& g, float** lut, size_t* bytes)
 {
     *bytes = 0;
-    if ((fmt == kNV12 || fmt == kP016) && !deep) {
-        const int n = fmt == kNV12 ? 256 : 1024, shift = fmt == kNV12 ? 0 : 6;
+    if (format_is_yuv(fmt) && !deep) {
+        const bool b16 = format_is_yuv16(fmt);
+        const int n = b16 ? 1024 : 256, shift = b16 ? 6 : 0;
         const size_t b = (size_t)2 * n * n * sizeof(float);
         cudaError_t e = cudaMalloc(lut, b);
         if (e != cudaSuccess) return e;
@@ -254,10 +263,10 @@ static cudaError_t build_side_lut(int fmt, bool deep, Geo& g, float** lut, size_
 // the distorted description of ssimu2_create_mixed (checked like ssimu2_config, before any device call)
 static int check_source(const ssimu2_source* s)
 {
-    if (s->format < 0 || s->format > kLINEARF32) return SSIMU2_E_UNSUPPORTED;
+    if (!format_known(s->format)) return SSIMU2_E_UNSUPPORTED;
     if (s->matrix < 0 || s->matrix > 2) return SSIMU2_E_UNSUPPORTED;
     if (s->flags & ~SSIMU2_FLAG_P016_DEEP) return SSIMU2_E_UNSUPPORTED;
-    if ((s->flags & SSIMU2_FLAG_P016_DEEP) && s->format != kP016) return SSIMU2_E_UNSUPPORTED;
+    if ((s->flags & SSIMU2_FLAG_P016_DEEP) && !format_is_yuv16(s->format)) return SSIMU2_E_UNSUPPORTED;
     for (int i = 0; i < 4; i++)
         if (s->reserved[i]) return SSIMU2_E_INVALID;
     return SSIMU2_OK;
@@ -267,7 +276,7 @@ static int check_source(const ssimu2_source* s)
 // mean nothing to the packed formats.
 static bool same_source(const ssimu2_config* cfg, const ssimu2_source* s)
 {
-    const bool yuv = cfg->format == kNV12 || cfg->format == kP016;
+    const bool yuv = format_is_yuv(cfg->format);
     return s->format == cfg->format && (s->flags & SSIMU2_FLAG_P016_DEEP) == (cfg->flags & SSIMU2_FLAG_P016_DEEP) &&
            (!yuv || (s->matrix == cfg->matrix && (s->full_range != 0) == (cfg->full_range != 0)));
 }
@@ -335,7 +344,7 @@ static void launch_frontend_kernel(const Geo& g, Slot& sl, uint32_t frame0, uint
     k_frontend2<FMT, SIDE><<<dim3((rx + per_cta - 1) / per_cta, ry, n), kF2Threads, 0, sl.stream>>>(g, sl.in_d, sl.xyb, (int)frame0);
 }
 
-// fe_fmt: the front-end format of the side(s) (kP016A for P016 with SSIMU2_FLAG_P016_DEEP)
+// fe_fmt: the front-end format of the side(s) (kP016A / kP216A / kYUV444P16A for a 16-bit YUV side with SSIMU2_FLAG_P016_DEEP)
 template <int SIDE>
 static int launch_frontend_side(const Geo& g, int fe_fmt, Slot& sl, uint32_t frame0, uint32_t n)
 {
@@ -347,6 +356,12 @@ static int launch_frontend_side(const Geo& g, int fe_fmt, Slot& sl, uint32_t fra
     case kSRGB16: launch_frontend_kernel<kSRGB16, SIDE>(g, sl, frame0, n); break;
     case kSRGBF32: launch_frontend_kernel<kSRGBF32, SIDE>(g, sl, frame0, n); break;
     case kLINEARF32: launch_frontend_kernel<kLINEARF32, SIDE>(g, sl, frame0, n); break;
+    case kNV16: launch_frontend_kernel<kNV16, SIDE>(g, sl, frame0, n); break;
+    case kP216: launch_frontend_kernel<kP216, SIDE>(g, sl, frame0, n); break;
+    case kP216A: launch_frontend_kernel<kP216A, SIDE>(g, sl, frame0, n); break;
+    case kYUV444: launch_frontend_kernel<kYUV444, SIDE>(g, sl, frame0, n); break;
+    case kYUV444P16: launch_frontend_kernel<kYUV444P16, SIDE>(g, sl, frame0, n); break;
+    case kYUV444P16A: launch_frontend_kernel<kYUV444P16A, SIDE>(g, sl, frame0, n); break;
     default: return SSIMU2_E_UNSUPPORTED;
     }
     return 0;
@@ -498,7 +513,7 @@ static int finish_pair(ssimu2_handle* h)
     return 0;
 }
 
-static bool is_yuv(int fmt) { return fmt == kNV12 || fmt == kP016; }
+static bool is_yuv(int fmt) { return format_is_yuv(fmt); }
 
 // side 0: a reference frame, 1: a distorted frame (each side is checked against its own format); host frames with the byte
 // count copied from plane[0]
@@ -591,7 +606,7 @@ static int submit_host_pair(ssimu2_handle* h, const ssimu2_frame* ref, size_t re
 
 extern "C" {
 
-uint32_t ssimu2_version(void) { return (2u << 16) | 2u; }
+uint32_t ssimu2_version(void) { return (2u << 16) | 3u; }
 
 const char* ssimu2_strerror(int status)
 {
@@ -615,11 +630,11 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
     if (!out || !cfg) return SSIMU2_E_INVALID;
     *out = nullptr;
     if (cfg->width < 8 || cfg->height < 8 || cfg->width > 32768 || cfg->height > 32768) return SSIMU2_E_UNSUPPORTED;
-    if (cfg->format < 0 || cfg->format > kLINEARF32) return SSIMU2_E_UNSUPPORTED;
+    if (!format_known(cfg->format)) return SSIMU2_E_UNSUPPORTED;
     if (cfg->matrix < 0 || cfg->matrix > 2) return SSIMU2_E_UNSUPPORTED;
     if (cfg->pipeline > SSIMU2_PIPELINE_SPLIT) return SSIMU2_E_UNSUPPORTED;
     if (cfg->flags & ~(SSIMU2_FLAG_SCORE_ONLY | SSIMU2_FLAG_NO_TIMING | SSIMU2_FLAG_P016_DEEP)) return SSIMU2_E_UNSUPPORTED;
-    if ((cfg->flags & SSIMU2_FLAG_P016_DEEP) && cfg->format != kP016) return SSIMU2_E_UNSUPPORTED;
+    if ((cfg->flags & SSIMU2_FLAG_P016_DEEP) && !format_is_yuv16(cfg->format)) return SSIMU2_E_UNSUPPORTED;
     if ((cfg->flags & SSIMU2_FLAG_SCORE_ONLY) && cfg->pipeline != SSIMU2_PIPELINE_DEFAULT) return SSIMU2_E_UNSUPPORTED;
     for (int i = 0; i < 5; i++)
         if (cfg->reserved[i]) return SSIMU2_E_INVALID;
@@ -646,8 +661,8 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
     const bool deep_dis = h->mixed ? (dis->flags & SSIMU2_FLAG_P016_DEEP) != 0 : deep_ref;
     h->fmt[0] = cfg->format;
     h->fmt[1] = h->mixed ? dis->format : cfg->format;
-    h->fe_fmt[0] = deep_ref ? kP016A : h->fmt[0];
-    h->fe_fmt[1] = deep_dis ? kP016A : h->fmt[1];
+    h->fe_fmt[0] = deep_ref ? deep_fe_fmt(h->fmt[0]) : h->fmt[0];
+    h->fe_fmt[1] = deep_dis ? deep_fe_fmt(h->fmt[1]) : h->fmt[1];
     h->ring = cfg->ring ? cfg->ring : kDefaultRing;
     if (h->ring > 16) h->ring = 16;
     h->batch = cfg->batch ? cfg->batch : kDefaultBatch;

@@ -16,7 +16,7 @@ from __future__ import annotations
 from dataclasses import dataclass
 from typing import Iterable, List, Optional, Sequence, Tuple
 
-from .ssimulacra2 import ColorMatrix, DeviceFrame, PixelFormat, ShardedSsimulacra2, Ssimulacra2
+from .ssimulacra2 import YUV16_FORMATS, ColorMatrix, DeviceFrame, PixelFormat, ShardedSsimulacra2, Ssimulacra2
 
 
 @dataclass
@@ -106,14 +106,14 @@ class TurboMetrics:
                  dis_full_range: Optional[bool] = None, dis_bit_depth: Optional[int] = None):
         """score_only: the engine only ever hands out scores (`FrameScores`), so it asks the scorer for nothing else
         (SSIMU2_FLAG_SCORE_ONLY: same score bits, ~8 % faster).  bit_depth: of the decoded stream (the reference reads it from the
-        stream's colour info, turbo-metrics/src/lib.rs:185-199); P016 frames of a stream deeper than 10 bits select the
+        stream's colour info, turbo-metrics/src/lib.rs:185-199); P016 / P216 / YUV444P16 frames of a stream deeper than 10 bits select the
         front-end without the 10-bit memo tables (SSIMU2_FLAG_P016_DEEP).
         dis_fmt, dis_matrix, dis_full_range, dis_bit_depth: the distorted source's own frame format and colour characteristics
         (None = as the reference), the `compute_one(fref, cc_ref, fdis, cc_dis)` shape of lib.rs:268-360; `bit_depth` then
         applies to the reference side and `dis_bit_depth` to the distorted side."""
-        deep = fmt == PixelFormat.P016 and bit_depth is not None and bit_depth > 10
+        deep = fmt in YUV16_FORMATS and bit_depth is not None and bit_depth > 10
         dfmt = fmt if dis_fmt is None else dis_fmt
-        dis_deep = None if dis_bit_depth is None else (dfmt == PixelFormat.P016 and dis_bit_depth > 10)
+        dis_deep = None if dis_bit_depth is None else (dfmt in YUV16_FORMATS and dis_bit_depth > 10)
         self.ssimulacra2 = Ssimulacra2(width, height, fmt, matrix, full_range, device, batch, ring, score_only=score_only,
                                        p016_deep=deep, dis_fmt=dis_fmt, dis_matrix=dis_matrix, dis_full_range=dis_full_range,
                                        dis_p016_deep=dis_deep)

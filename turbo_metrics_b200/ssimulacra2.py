@@ -30,6 +30,16 @@ class PixelFormat(IntEnum):
     SRGB16 = 3
     SRGBF32 = 4
     LINEARF32 = 5
+    # NVDEC's 4:2:2 / 4:4:4 surfaces (cudaVideoSurfaceFormat_NV16 / _P216 / _YUV444 / _YUV444_16Bit)
+    NV16 = 8
+    P216 = 9
+    YUV444 = 10
+    YUV444P16 = 11
+
+
+YUV_FORMATS = (PixelFormat.NV12, PixelFormat.P016, PixelFormat.NV16, PixelFormat.P216, PixelFormat.YUV444, PixelFormat.YUV444P16)
+# the formats SSIMU2_FLAG_P016_DEEP applies to
+YUV16_FORMATS = (PixelFormat.P016, PixelFormat.P216, PixelFormat.YUV444P16)
 
 
 class ColorMatrix(IntEnum):
@@ -63,6 +73,20 @@ class DeviceFrame:
         base = buf.data_ptr() if hasattr(buf, "data_ptr") else buf.ctypes.data
         nbytes = buf.numel() * buf.element_size() if hasattr(buf, "numel") else buf.nbytes
         return DeviceFrame(base, base + pitch * coded_height, pitch, buf, nbytes)
+
+    @staticmethod
+    def yuv422(buf, pitch: int, coded_height: int) -> "DeviceFrame":
+        """NVDEC NV16 / P216 layout: Y at buf, interleaved CbCr of full height at buf + pitch*coded_height.
+        buf: 1-D uint8 torch tensor (device or pinned host) or numpy array.  `nbytes` (what compute_from_cpu copies) is the
+        buffer's size, which must reach the end of the last chroma row."""
+        return DeviceFrame.yuv420(buf, pitch, coded_height)
+
+    @staticmethod
+    def yuv444(buf, pitch: int, coded_height: int) -> "DeviceFrame":
+        """NVDEC YUV444 / YUV444_16Bit layout: Y, Cb and Cr planes of `coded_height` rows at `pitch` bytes, one after the other
+        (also a contiguous (3, coded_height, pitch) array).  The library finds Cr at plane1 + (plane1 - plane0).
+        buf: 1-D uint8 torch tensor (device or pinned host) or numpy array."""
+        return DeviceFrame.yuv420(buf, pitch, coded_height)
 
     @staticmethod
     def packed(img, pitch: Optional[int] = None) -> "DeviceFrame":
@@ -105,7 +129,7 @@ def make_source(cfg: Config, dis_fmt=None, dis_matrix=None, dis_full_range=None,
     src.matrix = int(cfg.matrix if dis_matrix is None else dis_matrix)
     src.full_range = int(cfg.full_range if dis_full_range is None else dis_full_range)
     if dis_p016_deep is None:
-        dis_p016_deep = bool(cfg.flags & _lib.FLAG_P016_DEEP) and src.format == PixelFormat.P016
+        dis_p016_deep = bool(cfg.flags & _lib.FLAG_P016_DEEP) and src.format in YUV16_FORMATS
     src.flags = _lib.FLAG_P016_DEEP if dis_p016_deep else 0
     return src
 
@@ -116,7 +140,7 @@ def is_mixed(cfg: Config, src: Optional[Source]) -> bool:
     if src is None:
         return False
     deep = _lib.FLAG_P016_DEEP
-    yuv = cfg.format in (PixelFormat.NV12, PixelFormat.P016)
+    yuv = cfg.format in YUV_FORMATS
     return not (src.format == cfg.format and (src.flags & deep) == (cfg.flags & deep) and
                 (not yuv or (src.matrix == cfg.matrix and bool(src.full_range) == bool(cfg.full_range))))
 
@@ -134,7 +158,7 @@ class Ssimulacra2:
         pipeline with the H-pass planes in HBM (debug_read(what=1)).
         score_only: SSIMU2_FLAG_SCORE_ONLY -- skip the work whose weights are zero (scores identical, no norms).
         input_group: pairs per front-end launch (0 = whole batch): input frames are consumed sooner, see wait_input().
-        p016_deep: SSIMU2_FLAG_P016_DEEP -- P016 samples with more than 10 significant bits (12-bit sources): same results,
+        p016_deep: SSIMU2_FLAG_P016_DEEP -- P016 / P216 / YUV444P16 samples with more than 10 significant bits (12-bit sources): same results,
         a front-end without the 10-bit memo tables (of the reference frames when the distorted frames are described apart).
         dis_fmt, dis_matrix, dis_full_range, dis_p016_deep: the distorted frames' own description (None = as the reference);
         any of them set creates the handle with ssimu2_create_mixed.  Host frames of a mixed handle are copied with each

@@ -8,6 +8,8 @@ There is no network, so datasets and bitstreams are replaced by seeded procedura
 Layouts match what the decoder / NPP would hand over:
   yuv420 : NVDEC biplanar buffer, Y rows at `pitch` bytes, interleaved CbCr at pitch*coded_height
            (cudarse-video/src/dec.rs:299-366); 8-bit (NV12) or 10-bit in the high bits of u16 (P016)
+  yuv422 : the same with an interleaved CbCr plane of full height (NV16 / P216)
+  yuv444 : Y, Cb, Cr planes of coded_height rows one after the other (YUV444 / YUV444P16)
   srgb8  : packed RGB u8, (H, W, 3)
 Everything is torch so the same code runs on the CPU (tests, oracle inputs) and on the GPU (bench).
 """
@@ -110,6 +112,71 @@ def make_pair_yuv420(w: int, h: int, bits: int = 8, frame: int = 0, seed: int = 
     cr_d = _distort(cr, g, device, 0.75 / 255.0, q)
     pitch, coded_h, _ = yuv420_geometry(w, h, bits)
     return (_pack_yuv(lum, cb, cr, w, h, bits, device), _pack_yuv(lum_d, cb_d, cr_d, w, h, bits, device), pitch, coded_h)
+
+
+def yuv_geometry(w: int, h: int, bits: int, sub: str):
+    """yuv420_geometry for sub = "420", "422" or "444": (pitch, coded_height, total bytes) of an NVDEC-like surface."""
+    pitch, coded_h, total = yuv420_geometry(w, h, bits)
+    if sub == "420":
+        return pitch, coded_h, total
+    return pitch, coded_h, pitch * coded_h * (2 if sub == "422" else 3)
+
+
+def quantize_yuv(yv, cb, cr, bits: int):
+    """[0,1] floats -> limited-range integer samples: 8-bit codes, or 10-bit codes in the high bits of u16 (int32 tensors)."""
+    if bits == 8:
+        return (torch.round(16 + 219 * yv).clamp(0, 255).to(torch.int32),
+                torch.round(128 + 224 * (cb - 0.5)).clamp(0, 255).to(torch.int32),
+                torch.round(128 + 224 * (cr - 0.5)).clamp(0, 255).to(torch.int32))
+    return (torch.round(64 + 876 * yv).clamp(0, 1023).to(torch.int32) << 6,
+            torch.round(512 + 896 * (cb - 0.5)).clamp(0, 1023).to(torch.int32) << 6,
+            torch.round(512 + 896 * (cr - 0.5)).clamp(0, 1023).to(torch.int32) << 6)
+
+
+def pack_yuv_samples(yq, cbq, crq, w: int, h: int, bits: int, sub: str, pitch: int, coded_h: int, device="cpu"):
+    """Integer samples -> NVDEC-like surface (1-D uint8): Y (h, w); Cb / Cr (h, ceil(w/2)) for "422", (h, w) for "444".
+    4:2:2: interleaved CbCr plane at pitch*coded_h; 4:4:4: Cb plane there, Cr plane at 2*pitch*coded_h."""
+    bps = 1 if bits == 8 else 2
+    n = pitch * coded_h * (2 if sub == "422" else 3) // bps
+    buf = torch.zeros(n, dtype=torch.int32, device=device)
+    p = pitch // bps
+    plane = p * coded_h
+    buf[: p * h].view(h, p)[:, :w] = yq
+    if sub == "422":
+        cw = (w + 1) // 2
+        uv = buf[plane: plane + p * h].view(h, p)
+        uv[:, 0:2 * cw:2] = cbq
+        uv[:, 1:2 * cw:2] = crq
+    else:
+        buf[plane: plane + p * h].view(h, p)[:, :w] = cbq
+        buf[2 * plane: 2 * plane + p * h].view(h, p)[:, :w] = crq
+    if bits == 8:
+        return buf.to(torch.uint8)
+    lo = (buf & 0xFF).to(torch.uint8)
+    hi = ((buf >> 8) & 0xFF).to(torch.uint8)
+    return torch.stack([lo, hi], dim=1).reshape(-1).contiguous()
+
+
+def make_pair_yuv(w: int, h: int, bits: int = 8, sub: str = "444", frame: int = 0, seed: int = 1, device="cpu"):
+    """make_pair_yuv420's content with chroma at 4:2:2 ("422": ceil(w/2) x h) or 4:4:4 ("444": w x h) resolution.
+    -> (ref_buf, dis_buf, pitch, coded_height); buffers are 1-D uint8 tensors on `device` (NV16 / P216 / YUV444 / YUV444P16)."""
+    assert sub in ("422", "444")
+    g = _gen(seed, frame, device)
+    ch, cw = h, (w + 1) // 2 if sub == "422" else w
+    lum = _base_luma(h, w, frame, g, device)
+    yy = torch.arange(ch, device=device, dtype=torch.float32)[:, None] / max(ch - 1, 1)
+    xx = torch.arange(cw, device=device, dtype=torch.float32)[None, :] / max(cw - 1, 1)
+    cb = 0.5 + 0.2 * (xx - 0.5) * 2 * torch.cos(2 * math.pi * (yy + frame / 131.0)) + 0.05 * _smooth_noise(ch, cw, 8, g, device)
+    cr = 0.5 + 0.2 * (yy - 0.5) * 2 * torch.sin(2 * math.pi * (xx + frame / 171.0)) + 0.05 * _smooth_noise(ch, cw, 8, g, device)
+    cb, cr = cb.clamp(0, 1), cr.clamp(0, 1)
+    q = 4.0 / 219.0
+    lum_d = _distort(lum, g, device, 1.5 / 255.0, q)
+    cb_d = _distort(cb, g, device, 0.75 / 255.0, q)
+    cr_d = _distort(cr, g, device, 0.75 / 255.0, q)
+    pitch, coded_h, _ = yuv_geometry(w, h, bits, sub)
+    ref = pack_yuv_samples(*quantize_yuv(lum, cb, cr, bits), w, h, bits, sub, pitch, coded_h, device)
+    dis = pack_yuv_samples(*quantize_yuv(lum_d, cb_d, cr_d, bits), w, h, bits, sub, pitch, coded_h, device)
+    return ref, dis, pitch, coded_h
 
 
 def make_pair_srgb8(w: int, h: int, frame: int = 0, seed: int = 1, device="cpu"):
