@@ -46,7 +46,9 @@
  *     are not re-entrant; different handles may be driven from different threads.
  *   - Mixed sources: ssimu2_create_mixed binds the distorted frames to a description of their own (format, matrix, range),
  *     like TurboMetrics::compute_one(fref, cc_ref, fdis, cc_dis), which converts each frame with its own HwFrame variant and
- *     colour characteristics (turbo-metrics/src/lib.rs:268-360).  Both sides keep one width and height.
+ *     colour characteristics (turbo-metrics/src/lib.rs:268-360).  The distorted frames may also be smaller than the
+ *     reference (ssimu2_source.width / height: an encoding ladder's lower rungs against their source); they are upscaled
+ *     to the reference's size on the GPU with a fixed bicubic filter before they are scored (see ssimu2_source).
  *   - There is no CPU fallback: if no CUDA device is usable every entry point fails.
  */
 #ifndef SSIMU2_B200_H
@@ -153,7 +155,22 @@ typedef struct {
     int32_t matrix;       /* ssimu2_matrix (YUV formats) */
     int32_t full_range;   /* 0 = limited, 1 = full */
     uint32_t flags;       /* SSIMU2_FLAG_P016_DEEP only, and only with a 16-bit YUV format (P016, P216, YUV444P16) */
-    uint32_t reserved[4]; /* must be 0 */
+    /* Scaled distorted frames: the size of the distorted frames, 1 <= width <= cfg.width and 1 <= height <= cfg.height
+     * (a larger side is SSIMU2_E_UNSUPPORTED, one of the two 0 is SSIMU2_E_INVALID).  0, 0 = the reference's size.  The pair is
+     * scored at the reference's size: each distorted frame is first upscaled in its own sample domain to a frame of the same
+     * format at cfg.width x cfg.height, plane by plane on the plane's own grid (4:2:0 chroma ceil(width / 2) x ceil(height / 2)
+     * -> ceil(cfg.width / 2) x ceil(cfg.height / 2); 4:2:2 chroma ceil(width / 2) x height -> ceil(cfg.width / 2) x cfg.height;
+     * 4:4:4 chroma and packed RGB as luma; interleaved Cb / Cr and the three RGB channels each on their own).  The filter is
+     * separable bicubic Catmull-Rom (Keys, a = -0.5), centre-aligned (sx = (x + 0.5) * in / out - 0.5), clamp-to-edge, taps
+     * floor(sx) - 1 .. floor(sx) + 2, weights computed in double and rounded to float, evaluated in f32 horizontally first as
+     * a = w0 * s0 followed by three fmaf steps.  u8 / u16 results are rounded half to even and clamped to [0, 255] /
+     * [0, 65535] (16-bit results are not re-quantised to 10 bits); f32 results are stored unrounded and unclamped.  An axis
+     * whose size is unchanged is copied exactly.  This is NOT ffmpeg swscale's bicubic (B = 0, C = 0.6, fixed point): scores
+     * differ from those of an ffmpeg-upscaled pipeline by that difference.  Since ABI 2.3; ssimu2_version() is unchanged, so
+     * probe the capability by creating a handle: an older library returns SSIMU2_E_INVALID for these words.  Distorted frames
+     * are checked against the layout rule at their own size (host byte counts too). */
+    uint32_t width, height;
+    uint32_t reserved[2]; /* must be 0 */
 } ssimu2_source;
 
 /* ---- lifetime ------------------------------------------------------------------------ */
@@ -162,9 +179,12 @@ int ssimu2_create(ssimu2_t **out, const ssimu2_config *cfg);
  * SSIMU2_FLAG_P016_DEEP applies to the reference side only); dis == NULL: exactly ssimu2_create.  `dis` is checked before any
  * device call: a bad format or matrix, a flag other than SSIMU2_FLAG_P016_DEEP, or that flag with a format other than P016 / P216
  * / YUV444P16 is SSIMU2_E_UNSUPPORTED; non-zero reserved fields are SSIMU2_E_INVALID.  When the two sides are the same effective description
- * (same format and deep flag; for the YUV formats also the same matrix and range) the result is an ordinary handle: one
+ * (same format and deep flag; for the YUV formats also the same matrix and range; the same size) the result is an ordinary handle: one
  * front-end launch per input group and the same bits.  Otherwise the front-end runs once per side on the slot's stream, and
- * the frames of each side are checked against that side's format (ssimu2_frame pitch rule). */
+ * the frames of each side are checked against that side's format and size (ssimu2_frame pitch rule).  A scaled handle runs
+ * three kernels per input group: the reference's front-end, the upscale of the distorted frames into handle-owned staging
+ * memory (one frame of the distorted format at the reference's size per pair of an input group, per ring slot) and the
+ * distorted side's front-end.  Its io / alg bytes per pair count the distorted input at its own size. */
 int ssimu2_create_mixed(ssimu2_t **out, const ssimu2_config *cfg, const ssimu2_source *dis);
 int ssimu2_destroy(ssimu2_t *h);
 /* Device bytes owned by the handle (Ssimulacra2::mem_usage). */

@@ -27,9 +27,26 @@ class Config(C.Structure):
 
 
 class Source(C.Structure):
-    """ssimu2_source: the description of the distorted frames of a mixed handle (ssimu2_create_mixed)."""
+    """ssimu2_source: the description of the distorted frames of a mixed handle (ssimu2_create_mixed).  `width` and `height`
+    (the distorted frames' size, 0 = the reference's) are the C struct's first two of the four words `reserved` views."""
     _fields_ = [("format", C.c_int32), ("matrix", C.c_int32), ("full_range", C.c_int32), ("flags", C.c_uint32),
                 ("reserved", C.c_uint32 * 4)]
+
+    @property
+    def width(self) -> int:
+        return self.reserved[0]
+
+    @width.setter
+    def width(self, v: int):
+        self.reserved[0] = v
+
+    @property
+    def height(self) -> int:
+        return self.reserved[1]
+
+    @height.setter
+    def height(self, v: int):
+        self.reserved[1] = v
 
 
 PIPELINE_DEFAULT, PIPELINE_SPLIT = 0, 1

@@ -14,9 +14,12 @@
 #include "../../include/ssimu2_b200_debug.h"
 #include "frame_layout.h"
 #include "ssimu2_kernels.cuh"
+#include "resample.cuh"
 
 #include <cstdio>
 #include <cstdlib>
+#include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <new>
 #include <vector>
@@ -68,6 +71,9 @@ struct Slot {
     uint8_t* staging = nullptr;       // device staging for host frames: [batch][2][staging_frame_bytes]
     FramePair* in_h = nullptr;        // pinned frame table of the batch being recorded
     FramePair* in_d = nullptr;        // its device copy (uploaded per front-end launch)
+    uint8_t* rs_frames = nullptr;     // scaled handle: the upscaled distorted frames of one front-end launch [rs_group][rs.dst_stride]
+    FramePair* rs_in_h = nullptr;     // scaled handle: frame table of the distorted front-end (dis entries point at rs_frames)
+    FramePair* rs_in_d = nullptr;     // its device copy
     TmaMaps maps{};                   // tensor maps of this slot's H-pass / XYB buffers, per scale (V pass)
     TmaMapsH maps_h{};                // (H pass)
     TmaMapsX maps_x{};                // (fused H+V kernel)
@@ -94,6 +100,14 @@ struct ssimu2_handle {
     int fe_fmt[2] = {0, 0};           // their front-end formats (kP016A / kP216A / kYUV444P16A: with SSIMU2_FLAG_P016_DEEP)
     Geo geo_dis{};
     float* eotf_lut_dis = nullptr;
+    uint32_t side_w[2] = {0, 0}, side_h[2] = {0, 0};   // size of the reference / distorted frames
+    // scaled distorted frames (ssimu2_source.width / height smaller than the reference): k_resample upscales them into
+    // rs_frames before the distorted side's front-end; rs holds the plane grids and tap tables (rs_tab), rs_group is the
+    // most pairs one front-end launch covers
+    bool scaled = false;
+    RsArgs rs{};
+    void* rs_tab = nullptr;
+    uint32_t rs_group = 0;
     uint32_t batch = 0, ring = 0, input_group = 0;
     std::vector<Slot> slots;
     uint32_t cur = 0;
@@ -220,10 +234,12 @@ static void build_geo(ssimu2_handle* h)
     g.coef = make_coef(h->cfg.format, h->cfg.matrix, h->cfg.full_range);
     // SURVEY.md section 8(d): B_alg = 120*sum(P_s) + 2*in_0*P_0 + 72*sum_{s>=1}(P_s), in_0 = input bytes per pixel of the pair
     // (each side at its own bytes per pixel: in_bytes_per_px is per two images of one format)
-    const unsigned long long in2 = (unsigned long long)(in_bytes_per_px(h->fmt[0]) + in_bytes_per_px(h->fmt[1]));
-    h->alg_bytes = 120ULL * sum_px + in2 * h->cfg.width * h->cfg.height + 72ULL * sum_px_ge1;
+    // (a scaled distorted side counts at its own size)
+    const unsigned long long in2 = (unsigned long long)in_bytes_per_px(h->fmt[0]) * h->side_w[0] * h->side_h[0] +
+                                   (unsigned long long)in_bytes_per_px(h->fmt[1]) * h->side_w[1] * h->side_h[1];
+    h->alg_bytes = 120ULL * sum_px + in2 + 72ULL * sum_px_ge1;
     // compulsory I/O floor B_io = in_0 * P_0 + 8
-    h->io_bytes = in2 * h->cfg.width * h->cfg.height / 2 + 8ULL;
+    h->io_bytes = in2 / 2 + 8ULL;
 }
 
 // Exact memo of one side's transfer function (Geo::eotf_lut), built by the device code it replaces: the R / B tables of
@@ -261,16 +277,23 @@ static cudaError_t build_side_lut(int fmt, bool deep, Geo& g, float** lut, size_
 }
 
 // the distorted description of ssimu2_create_mixed (checked like ssimu2_config, before any device call)
-static int check_source(const ssimu2_source* s)
+static int check_source(const ssimu2_config* cfg, const ssimu2_source* s)
 {
     if (!format_known(s->format)) return SSIMU2_E_UNSUPPORTED;
     if (s->matrix < 0 || s->matrix > 2) return SSIMU2_E_UNSUPPORTED;
     if (s->flags & ~SSIMU2_FLAG_P016_DEEP) return SSIMU2_E_UNSUPPORTED;
     if ((s->flags & SSIMU2_FLAG_P016_DEEP) && !format_is_yuv16(s->format)) return SSIMU2_E_UNSUPPORTED;
-    for (int i = 0; i < 4; i++)
+    for (int i = 0; i < 2; i++)
         if (s->reserved[i]) return SSIMU2_E_INVALID;
+    if ((s->width == 0) != (s->height == 0)) return SSIMU2_E_INVALID;
+    // only upscaling: the distorted frames are at most the reference's size on each axis
+    if (s->width > cfg->width || s->height > cfg->height) return SSIMU2_E_UNSUPPORTED;
     return SSIMU2_OK;
 }
+
+// the distorted frames' size (0, 0: the reference's)
+static uint32_t source_width(const ssimu2_config* cfg, const ssimu2_source* s) { return s && s->width ? s->width : cfg->width; }
+static uint32_t source_height(const ssimu2_config* cfg, const ssimu2_source* s) { return s && s->height ? s->height : cfg->height; }
 
 // The two sides are one effective description: same format and deep flag, and (YUV) same matrix and range.  Matrix and range
 // mean nothing to the packed formats.
@@ -278,7 +301,101 @@ static bool same_source(const ssimu2_config* cfg, const ssimu2_source* s)
 {
     const bool yuv = format_is_yuv(cfg->format);
     return s->format == cfg->format && (s->flags & SSIMU2_FLAG_P016_DEEP) == (cfg->flags & SSIMU2_FLAG_P016_DEEP) &&
-           (!yuv || (s->matrix == cfg->matrix && (s->full_range != 0) == (cfg->full_range != 0)));
+           (!yuv || (s->matrix == cfg->matrix && (s->full_range != 0) == (cfg->full_range != 0))) &&
+           source_width(cfg, s) == cfg->width && source_height(cfg, s) == cfg->height;
+}
+
+// ---- scaled distorted frames: plane grids, tap tables and the staged layout of k_resample (resample.cuh) ----
+// Catmull-Rom (Keys, a = -0.5) weight of a tap at distance t, in double (this file's host code is built with
+// -ffp-contract=off: the oracle evaluates the same expressions uncontracted).
+static double keys_weight(double t)
+{
+    if (t < 1.0) return (1.5 * t - 2.5) * t * t + 1.0;
+    if (t < 2.0) return ((-0.5 * t + 2.5) * t - 4.0) * t + 2.0;
+    return 0.0;
+}
+
+// Taps of an axis of `in` -> `out` samples: output coordinate x reads source samples i - 1 .. i + 2 (clamped when read),
+// i = floor(sx), sx = (x + 0.5) * in / out - 0.5 (centre-aligned).  An axis of unchanged size gets (0, 1, 0, 0).
+static void axis_taps(int in, int out, float4* w, int* j0)
+{
+    const double scale = (double)in / (double)out;
+    for (int x = 0; x < out; x++) {
+        const double sx = (x + 0.5) * scale - 0.5;
+        const int i = (int)floor(sx);
+        float ww[4];
+        for (int k = 0; k < 4; k++) ww[k] = (float)keys_weight(fabs(sx - (double)(i - 1 + k)));
+        w[x] = make_float4(ww[0], ww[1], ww[2], ww[3]);
+        j0[x] = i - 1;
+    }
+}
+
+// The plane grids of the distorted format at its own size (in) and the reference's (out), the staged layout (NVDEC-like:
+// pitch and planes 256-byte aligned; 4:4:4 Cr at plane[1] + (plane[1] - plane[0])) and the tap tables in one device buffer.
+static cudaError_t build_resample(ssimu2_handle* h)
+{
+    const int fmt = h->fmt[1];
+    const int W = (int)h->side_w[0], H = (int)h->side_h[0], Wd = (int)h->side_w[1], Hd = (int)h->side_h[1];
+    const bool yuv = format_is_yuv(fmt), yuv444 = fmt == kYUV444 || fmt == kYUV444P16, yuv420 = fmt == kNV12 || fmt == kP016;
+    const uint64_t s = fmt == kSRGBF32 || fmt == kLINEARF32 ? 4 : (format_is_yuv16(fmt) || fmt == kSRGB16) ? 2 : 1;
+    RsArgs& a = h->rs;
+    a.nplanes = !yuv ? 1 : yuv444 ? 3 : 2;
+    int dims[3][4];   // per plane: in_w, in_h, out_w, out_h (per channel)
+    int nch[3] = {yuv ? 1 : 3, yuv444 ? 1 : 2, 1};
+    dims[0][0] = Wd; dims[0][1] = Hd; dims[0][2] = W; dims[0][3] = H;
+    if (yuv444) {
+        for (int p = 1; p < 3; p++) memcpy(dims[p], dims[0], sizeof(dims[0]));
+    } else if (yuv) {
+        dims[1][0] = (Wd + 1) / 2; dims[1][1] = yuv420 ? (Hd + 1) / 2 : Hd;
+        dims[1][2] = (W + 1) / 2;  dims[1][3] = yuv420 ? (H + 1) / 2 : H;
+    }
+    uint64_t row = (uint64_t)W * nch[0] * s;
+    if (yuv) row = std::max<uint64_t>(row, (uint64_t)dims[1][2] * nch[1] * s);
+    a.dst_pitch = (uint32_t)((row + 255) / 256 * 256);
+    uint64_t off = 0;
+    for (int p = 0; p < a.nplanes; p++) {
+        a.pl[p].dst_off = (long long)off;
+        off += (uint64_t)a.dst_pitch * dims[p][3];
+        off = (off + 255) / 256 * 256;
+    }
+    a.dst_stride = (long long)off;
+    // 4:4:4: the front-end finds Cr at plane[1] + (plane[1] - plane[0]), so the three planes must be equally spaced
+    if (yuv444 && a.pl[2].dst_off != 2 * a.pl[1].dst_off) return cudaErrorInvalidValue;
+    // tap tables: per plane grid, x then y (4:4:4 chroma shares the luma tables)
+    std::vector<float4> w;
+    std::vector<int> j;
+    size_t wofs[3][2], jofs[3][2];
+    const int ngrids = yuv444 ? 1 : a.nplanes;
+    for (int p = 0; p < ngrids; p++)
+        for (int ax = 0; ax < 2; ax++) {
+            const int in = dims[p][ax], out = dims[p][2 + ax];
+            wofs[p][ax] = w.size();
+            jofs[p][ax] = j.size();
+            w.resize(w.size() + out);
+            j.resize(j.size() + out);
+            axis_taps(in, out, &w[wofs[p][ax]], &j[jofs[p][ax]]);
+        }
+    const size_t wb = w.size() * sizeof(float4), jb = j.size() * sizeof(int);
+    cudaError_t e = cudaMalloc(&h->rs_tab, wb + jb);
+    if (e != cudaSuccess) return e;
+    if ((e = cudaMemcpy(h->rs_tab, w.data(), wb, cudaMemcpyHostToDevice)) != cudaSuccess) return e;
+    if ((e = cudaMemcpy((uint8_t*)h->rs_tab + wb, j.data(), jb, cudaMemcpyHostToDevice)) != cudaSuccess) return e;
+    h->device_bytes += wb + jb;
+    const float4* wd = (const float4*)h->rs_tab;
+    const int* jd = (const int*)((uint8_t*)h->rs_tab + wb);
+    int tiles = 0;
+    for (int p = 0; p < a.nplanes; p++) {
+        RsPlane& P = a.pl[p];
+        const int g = yuv444 ? 0 : p;
+        P.in_w = dims[p][0]; P.in_h = dims[p][1]; P.out_w = dims[p][2]; P.out_h = dims[p][3];
+        P.x = RsAxis{wd + wofs[g][0], jd + jofs[g][0]};
+        P.y = RsAxis{wd + wofs[g][1], jd + jofs[g][1]};
+        P.tiles_x = (P.out_w + kRsTileX - 1) / kRsTileX;
+        P.tile0 = tiles;
+        tiles += P.tiles_x * ((P.out_h + kRsTileY - 1) / kRsTileY);
+    }
+    a.tiles = tiles;
+    return cudaSuccess;
 }
 
 // ---- TMA tensor maps (driver entry point fetched through the runtime; libcuda is not linked) ----
@@ -337,37 +454,66 @@ static int build_tma_maps(ssimu2_handle* h, Slot& sl)
 // k_hv + k_finalize (or k_hpass + k_vpass + k_finalize), then the D2H copy of scores and norms.
 
 template <int FMT, int SIDE>
-static void launch_frontend_kernel(const Geo& g, Slot& sl, uint32_t frame0, uint32_t n)
+static void launch_frontend_kernel(const Geo& g, const FramePair* tab, Slot& sl, uint32_t frame0, uint32_t n)
 {
     const int rx = (g.sc[0].w + kF2Region - 1) / kF2Region, ry = (g.sc[0].h + kF2Region - 1) / kF2Region;
     const int per_cta = (kF2Threads / 32) * f2_regions_per_warp(SIDE);
-    k_frontend2<FMT, SIDE><<<dim3((rx + per_cta - 1) / per_cta, ry, n), kF2Threads, 0, sl.stream>>>(g, sl.in_d, sl.xyb, (int)frame0);
+    k_frontend2<FMT, SIDE><<<dim3((rx + per_cta - 1) / per_cta, ry, n), kF2Threads, 0, sl.stream>>>(g, tab, sl.xyb, (int)frame0);
 }
 
-// fe_fmt: the front-end format of the side(s) (kP016A / kP216A / kYUV444P16A for a 16-bit YUV side with SSIMU2_FLAG_P016_DEEP)
+// fe_fmt: the front-end format of the side(s) (kP016A / kP216A / kYUV444P16A for a 16-bit YUV side with SSIMU2_FLAG_P016_DEEP);
+// tab: the device frame table the launch reads
 template <int SIDE>
-static int launch_frontend_side(const Geo& g, int fe_fmt, Slot& sl, uint32_t frame0, uint32_t n)
+static int launch_frontend_side(const Geo& g, int fe_fmt, const FramePair* tab, Slot& sl, uint32_t frame0, uint32_t n)
 {
     switch (fe_fmt) {
-    case kNV12: launch_frontend_kernel<kNV12, SIDE>(g, sl, frame0, n); break;
-    case kP016: launch_frontend_kernel<kP016, SIDE>(g, sl, frame0, n); break;
-    case kP016A: launch_frontend_kernel<kP016A, SIDE>(g, sl, frame0, n); break;
-    case kSRGB8: launch_frontend_kernel<kSRGB8, SIDE>(g, sl, frame0, n); break;
-    case kSRGB16: launch_frontend_kernel<kSRGB16, SIDE>(g, sl, frame0, n); break;
-    case kSRGBF32: launch_frontend_kernel<kSRGBF32, SIDE>(g, sl, frame0, n); break;
-    case kLINEARF32: launch_frontend_kernel<kLINEARF32, SIDE>(g, sl, frame0, n); break;
-    case kNV16: launch_frontend_kernel<kNV16, SIDE>(g, sl, frame0, n); break;
-    case kP216: launch_frontend_kernel<kP216, SIDE>(g, sl, frame0, n); break;
-    case kP216A: launch_frontend_kernel<kP216A, SIDE>(g, sl, frame0, n); break;
-    case kYUV444: launch_frontend_kernel<kYUV444, SIDE>(g, sl, frame0, n); break;
-    case kYUV444P16: launch_frontend_kernel<kYUV444P16, SIDE>(g, sl, frame0, n); break;
-    case kYUV444P16A: launch_frontend_kernel<kYUV444P16A, SIDE>(g, sl, frame0, n); break;
+    case kNV12: launch_frontend_kernel<kNV12, SIDE>(g, tab, sl, frame0, n); break;
+    case kP016: launch_frontend_kernel<kP016, SIDE>(g, tab, sl, frame0, n); break;
+    case kP016A: launch_frontend_kernel<kP016A, SIDE>(g, tab, sl, frame0, n); break;
+    case kSRGB8: launch_frontend_kernel<kSRGB8, SIDE>(g, tab, sl, frame0, n); break;
+    case kSRGB16: launch_frontend_kernel<kSRGB16, SIDE>(g, tab, sl, frame0, n); break;
+    case kSRGBF32: launch_frontend_kernel<kSRGBF32, SIDE>(g, tab, sl, frame0, n); break;
+    case kLINEARF32: launch_frontend_kernel<kLINEARF32, SIDE>(g, tab, sl, frame0, n); break;
+    case kNV16: launch_frontend_kernel<kNV16, SIDE>(g, tab, sl, frame0, n); break;
+    case kP216: launch_frontend_kernel<kP216, SIDE>(g, tab, sl, frame0, n); break;
+    case kP216A: launch_frontend_kernel<kP216A, SIDE>(g, tab, sl, frame0, n); break;
+    case kYUV444: launch_frontend_kernel<kYUV444, SIDE>(g, tab, sl, frame0, n); break;
+    case kYUV444P16: launch_frontend_kernel<kYUV444P16, SIDE>(g, tab, sl, frame0, n); break;
+    case kYUV444P16A: launch_frontend_kernel<kYUV444P16A, SIDE>(g, tab, sl, frame0, n); break;
+    default: return SSIMU2_E_UNSUPPORTED;
+    }
+    return 0;
+}
+
+template <int FMT>
+static void launch_resample_kernel(const RsArgs& a, Slot& sl, uint32_t frame0, uint32_t n)
+{
+    k_resample<FMT><<<dim3((unsigned)a.tiles, 1, n), kRsThreads, 0, sl.stream>>>(a, sl.in_d, (int)frame0);
+}
+
+// upscale the distorted frames of pairs [frame0, frame0 + n) into the slot's rs_frames (staged frame i - frame0 for pair i)
+static int launch_resample(const ssimu2_handle* h, Slot& sl, uint32_t frame0, uint32_t n)
+{
+    RsArgs a = h->rs;
+    a.dst = sl.rs_frames;
+    switch (h->fmt[1]) {
+    case kNV12: launch_resample_kernel<kNV12>(a, sl, frame0, n); break;
+    case kP016: launch_resample_kernel<kP016>(a, sl, frame0, n); break;
+    case kSRGB8: launch_resample_kernel<kSRGB8>(a, sl, frame0, n); break;
+    case kSRGB16: launch_resample_kernel<kSRGB16>(a, sl, frame0, n); break;
+    case kSRGBF32: launch_resample_kernel<kSRGBF32>(a, sl, frame0, n); break;
+    case kLINEARF32: launch_resample_kernel<kLINEARF32>(a, sl, frame0, n); break;
+    case kNV16: launch_resample_kernel<kNV16>(a, sl, frame0, n); break;
+    case kP216: launch_resample_kernel<kP216>(a, sl, frame0, n); break;
+    case kYUV444: launch_resample_kernel<kYUV444>(a, sl, frame0, n); break;
+    case kYUV444P16: launch_resample_kernel<kYUV444P16>(a, sl, frame0, n); break;
     default: return SSIMU2_E_UNSUPPORTED;
     }
     return 0;
 }
 
 // front-end of pairs [sl.fe_pairs, upto) of the batch being recorded in `sl`: one launch, or on a mixed handle one per side
+// (on a scaled handle with k_resample between the two)
 static int launch_frontend(ssimu2_handle* h, Slot& sl, uint32_t upto, bool time_it)
 {
     const uint32_t f0 = sl.fe_pairs;
@@ -379,19 +525,33 @@ static int launch_frontend(ssimu2_handle* h, Slot& sl, uint32_t upto, bool time_
         sl.have_dep = false;
     }
     CU_TRY(cudaMemcpyAsync(sl.in_d + f0, sl.in_h + f0, (size_t)n * sizeof(FramePair), cudaMemcpyHostToDevice, sl.stream));
+    if (h->scaled) {
+        // the distorted front-end reads the upscaled frames: staged frame i - f0 for pair i (plane layout of h->rs)
+        if (n > h->rs_group) return SSIMU2_E_INTERNAL;
+        for (uint32_t i = f0; i < upto; i++) {
+            uint8_t* d = sl.rs_frames + (size_t)(i - f0) * h->rs.dst_stride;
+            sl.rs_in_h[i] = sl.in_h[i];
+            sl.rs_in_h[i].dis.p0 = d;
+            sl.rs_in_h[i].dis.p1 = h->rs.nplanes > 1 ? d + h->rs.pl[1].dst_off : nullptr;
+            sl.rs_in_h[i].dis.pitch = h->rs.dst_pitch;
+            sl.rs_in_h[i].dis.pad = 0;
+        }
+        CU_TRY(cudaMemcpyAsync(sl.rs_in_d + f0, sl.rs_in_h + f0, (size_t)n * sizeof(FramePair), cudaMemcpyHostToDevice, sl.stream));
+    }
     if (time_it) cudaEventRecord(sl.ev_k[0], sl.stream);
     int r;
     if (!h->mixed) {
-        r = launch_frontend_side<kF2Both>(h->geo, h->fe_fmt[0], sl, f0, n);
+        r = launch_frontend_side<kF2Both>(h->geo, h->fe_fmt[0], sl.in_d, sl, f0, n);
     } else {
-        r = launch_frontend_side<kF2Ref>(h->geo, h->fe_fmt[0], sl, f0, n);
-        if (!r) r = launch_frontend_side<kF2Dis>(h->geo_dis, h->fe_fmt[1], sl, f0, n);
+        r = launch_frontend_side<kF2Ref>(h->geo, h->fe_fmt[0], sl.in_d, sl, f0, n);
+        if (!r && h->scaled) r = launch_resample(h, sl, f0, n);
+        if (!r) r = launch_frontend_side<kF2Dis>(h->geo_dis, h->fe_fmt[1], h->scaled ? sl.rs_in_d : sl.in_d, sl, f0, n);
     }
     if (r) return r;
     // the timing mark and the "inputs consumed" event follow the last launch: both sides have been read
     if (time_it) cudaEventRecord(sl.ev_k[1], sl.stream);
     CU_TRY(cudaGetLastError());
-    h->launches += h->mixed ? 2 : 1;
+    h->launches += !h->mixed ? 1 : h->scaled ? 3 : 2;
     if (sl.fe_launches >= sl.ev_fe.size()) {
         cudaEvent_t e = nullptr;
         CU_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -519,7 +679,7 @@ static bool is_yuv(int fmt) { return format_is_yuv(fmt); }
 // count copied from plane[0]
 static bool frame_ok(const ssimu2_handle* h, const ssimu2_frame* f, int side, bool host = false, size_t bytes = 0)
 {
-    return frame_layout_ok(h->fmt[side], h->cfg.width, h->cfg.height, f, host, bytes);
+    return frame_layout_ok(h->fmt[side], h->side_w[side], h->side_h[side], f, host, bytes);
 }
 
 // locate a ticket: 0 = results on host, 1 = in a launched slot, 2 = in the slot being filled
@@ -639,7 +799,7 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
     for (int i = 0; i < 5; i++)
         if (cfg->reserved[i]) return SSIMU2_E_INVALID;
     if (dis) {
-        const int rc = check_source(dis);
+        const int rc = check_source(cfg, dis);
         if (rc) return rc;
     }
     int ndev = 0;
@@ -657,8 +817,16 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
     if (!h) return SSIMU2_E_NOMEM;
     h->cfg = *cfg;
     h->mixed = dis != nullptr && !same_source(cfg, dis);
+    h->side_w[0] = cfg->width;
+    h->side_h[0] = cfg->height;
+    h->side_w[1] = source_width(cfg, dis);
+    h->side_h[1] = source_height(cfg, dis);
+    h->scaled = h->side_w[1] != cfg->width || h->side_h[1] != cfg->height;
     const bool deep_ref = (cfg->flags & SSIMU2_FLAG_P016_DEEP) != 0;
-    const bool deep_dis = h->mixed ? (dis->flags & SSIMU2_FLAG_P016_DEEP) != 0 : deep_ref;
+    // upscaled 16-bit samples generally have non-zero low bits: a scaled 16-bit YUV side always takes the deep front-end (the
+    // same bits as the memo path, which would send most samples to its arithmetic fall-back anyway)
+    const bool deep_dis = h->mixed ? (dis->flags & SSIMU2_FLAG_P016_DEEP) != 0 || (h->scaled && format_is_yuv16(dis->format))
+                                   : deep_ref;
     h->fmt[0] = cfg->format;
     h->fmt[1] = h->mixed ? dis->format : cfg->format;
     h->fe_fmt[0] = deep_ref ? deep_fe_fmt(h->fmt[0]) : h->fmt[0];
@@ -738,6 +906,10 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
         CR(build_side_lut(h->fmt[1], deep_dis, h->geo_dis, &h->eotf_lut_dis, &bytes));
         h->device_bytes += bytes;
     }
+    if (h->scaled) {
+        CR(build_resample(h));
+        h->rs_group = h->input_group ? h->input_group : h->batch;
+    }
     for (uint32_t i = 0; i < h->ring; i++) {
         Slot& sl = h->slots[i];
         const Geo& g = h->geo;
@@ -767,6 +939,13 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
         CR(cudaMallocHost(&sl.norms_h, (size_t)h->batch * 108 * sizeof(double)));
         CR(cudaMallocHost(&sl.scores_h, (size_t)h->batch * sizeof(double)));
         h->device_bytes += xyb_b + hb_b + hs_b + fl_b + part_b + in_b + (size_t)h->batch * 109 * sizeof(double);
+        if (h->scaled) {
+            const size_t rs_b = (size_t)h->rs_group * h->rs.dst_stride;
+            CR(cudaMalloc(&sl.rs_frames, rs_b));
+            CR(cudaMalloc(&sl.rs_in_d, in_b));
+            CR(cudaMallocHost(&sl.rs_in_h, in_b));
+            h->device_bytes += rs_b + in_b;
+        }
         rc = build_tma_maps(h, sl);
         if (rc) goto fail;
         sl.timed = (cfg->flags & SSIMU2_FLAG_NO_TIMING) == 0;
@@ -793,7 +972,9 @@ int ssimu2_destroy(ssimu2_t* h)
         for (cudaEvent_t e : sl.ev_fe) cudaEventDestroy(e);
         cudaFree(sl.xyb); cudaFree(sl.hb); cudaFree(sl.hstate); cudaFree(sl.hvflags); cudaFree(sl.partials);
         cudaFree(sl.norms_d); cudaFree(sl.scores_d); cudaFree(sl.staging); cudaFree(sl.in_d);
+        cudaFree(sl.rs_frames); cudaFree(sl.rs_in_d);
         if (sl.in_h) cudaFreeHost(sl.in_h);
+        if (sl.rs_in_h) cudaFreeHost(sl.rs_in_h);
         if (sl.norms_h) cudaFreeHost(sl.norms_h);
         if (sl.scores_h) cudaFreeHost(sl.scores_h);
         if (sl.stream) cudaStreamDestroy(sl.stream);
@@ -801,6 +982,7 @@ int ssimu2_destroy(ssimu2_t* h)
     cudaFree(h->scores_ring_d);
     cudaFree(h->eotf_lut);
     cudaFree(h->eotf_lut_dis);
+    cudaFree(h->rs_tab);
     delete h;
     return SSIMU2_OK;
 }

@@ -156,9 +156,12 @@ int submit_common(ssimu2_shard* s, uint32_t n, const ssimu2_frame* refs, const s
     // every frame is checked here, before any is queued: a frame the worker rejected later would fail the whole shard
     const bool host = frame_bytes != 0;
     const int ref_fmt = s->cfg.format, dis_fmt = s->has_dis ? s->dis.format : s->cfg.format;
+    // distorted frames at their own size (ssimu2_source.width / height; 0 = the reference's)
+    const uint32_t dis_w = s->has_dis && s->dis.width ? s->dis.width : s->cfg.width;
+    const uint32_t dis_h = s->has_dis && s->dis.height ? s->dis.height : s->cfg.height;
     for (uint32_t i = 0; i < n; i++)
         if (!frame_layout_ok(ref_fmt, s->cfg.width, s->cfg.height, &refs[i], host, frame_bytes) ||
-            !frame_layout_ok(dis_fmt, s->cfg.width, s->cfg.height, &diss[i], host, dis_bytes ? dis_bytes : frame_bytes))
+            !frame_layout_ok(dis_fmt, dis_w, dis_h, &diss[i], host, dis_bytes ? dis_bytes : frame_bytes))
             return SSIMU2_E_INVALID;
     if (first_ticket) *first_ticket = s->next_global;
     uint32_t i = 0;

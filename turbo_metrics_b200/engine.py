@@ -103,20 +103,23 @@ class TurboMetrics:
     def __init__(self, width: int, height: int, fmt: PixelFormat, matrix: ColorMatrix = ColorMatrix.BT709,
                  full_range: bool = False, device: int = 0, batch: int = 0, ring: int = 0, score_only: bool = True,
                  bit_depth: Optional[int] = None, dis_fmt: Optional[PixelFormat] = None, dis_matrix: Optional[ColorMatrix] = None,
-                 dis_full_range: Optional[bool] = None, dis_bit_depth: Optional[int] = None):
+                 dis_full_range: Optional[bool] = None, dis_bit_depth: Optional[int] = None, dis_width: Optional[int] = None,
+                 dis_height: Optional[int] = None):
         """score_only: the engine only ever hands out scores (`FrameScores`), so it asks the scorer for nothing else
         (SSIMU2_FLAG_SCORE_ONLY: same score bits, ~8 % faster).  bit_depth: of the decoded stream (the reference reads it from the
         stream's colour info, turbo-metrics/src/lib.rs:185-199); P016 / P216 / YUV444P16 frames of a stream deeper than 10 bits select the
         front-end without the 10-bit memo tables (SSIMU2_FLAG_P016_DEEP).
         dis_fmt, dis_matrix, dis_full_range, dis_bit_depth: the distorted source's own frame format and colour characteristics
         (None = as the reference), the `compute_one(fref, cc_ref, fdis, cc_dis)` shape of lib.rs:268-360; `bit_depth` then
-        applies to the reference side and `dis_bit_depth` to the distorted side."""
+        applies to the reference side and `dis_bit_depth` to the distorted side.
+        dis_width, dis_height: the distorted source's frame size when it is a lower rung of an encoding ladder (smaller than
+        width x height): its frames are upscaled to the reference's size on the GPU before they are scored."""
         deep = fmt in YUV16_FORMATS and bit_depth is not None and bit_depth > 10
         dfmt = fmt if dis_fmt is None else dis_fmt
         dis_deep = None if dis_bit_depth is None else (dfmt in YUV16_FORMATS and dis_bit_depth > 10)
         self.ssimulacra2 = Ssimulacra2(width, height, fmt, matrix, full_range, device, batch, ring, score_only=score_only,
                                        p016_deep=deep, dis_fmt=dis_fmt, dis_matrix=dis_matrix, dis_full_range=dis_full_range,
-                                       dis_p016_deep=dis_deep)
+                                       dis_p016_deep=dis_deep, dis_width=dis_width, dis_height=dis_height)
         info = self.ssimulacra2.info()
         self.window = info.batch * info.ring
 
@@ -169,10 +172,13 @@ class ShardedTurboMetrics:
 
     def __init__(self, width: int, height: int, fmt: PixelFormat, devices: Sequence[int], matrix: ColorMatrix = ColorMatrix.BT709,
                  full_range: bool = False, batch: int = 0, ring: int = 0, score_only: bool = True,
-                 dis_fmt: Optional[PixelFormat] = None, dis_matrix: Optional[ColorMatrix] = None, dis_full_range: Optional[bool] = None):
-        """dis_fmt, dis_matrix, dis_full_range: the distorted source's own description (None = as the reference)."""
+                 dis_fmt: Optional[PixelFormat] = None, dis_matrix: Optional[ColorMatrix] = None, dis_full_range: Optional[bool] = None,
+                 dis_width: Optional[int] = None, dis_height: Optional[int] = None):
+        """dis_fmt, dis_matrix, dis_full_range: the distorted source's own description (None = as the reference); dis_width,
+        dis_height: its frame size when smaller than the reference's (upscaled on the GPU)."""
         self.sharded = ShardedSsimulacra2(width, height, fmt, devices, matrix, full_range, batch, ring, score_only,
-                                          dis_fmt=dis_fmt, dis_matrix=dis_matrix, dis_full_range=dis_full_range)
+                                          dis_fmt=dis_fmt, dis_matrix=dis_matrix, dis_full_range=dis_full_range,
+                                          dis_width=dis_width, dis_height=dis_height)
         self.chunk = max(1, (batch or 8) * len(devices))
         self.window = self.chunk * max(2, ring or 3)
 

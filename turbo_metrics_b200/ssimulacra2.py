@@ -118,11 +118,14 @@ def make_config(width, height, fmt, matrix=ColorMatrix.BT709, full_range=False, 
     return cfg
 
 
-def make_source(cfg: Config, dis_fmt=None, dis_matrix=None, dis_full_range=None, dis_p016_deep=None) -> Optional[Source]:
+def make_source(cfg: Config, dis_fmt=None, dis_matrix=None, dis_full_range=None, dis_p016_deep=None, dis_width=None,
+                dis_height=None) -> Optional[Source]:
     """ssimu2_source of the distorted frames for a handle whose reference frames `cfg` describes, or None when no dis_*
     argument is given.  A dis_* argument left at None takes the reference's value; the deep flag is the reference's when the
-    distorted frames are P016 too."""
-    if dis_fmt is None and dis_matrix is None and dis_full_range is None and dis_p016_deep is None:
+    distorted frames are P016 too.  dis_width / dis_height: the distorted frames' size when they are smaller than the
+    reference's (upscaled to it on the GPU); None or 0 = the reference's."""
+    if dis_fmt is None and dis_matrix is None and dis_full_range is None and dis_p016_deep is None and \
+            dis_width is None and dis_height is None:
         return None
     src = Source()
     src.format = int(cfg.format if dis_fmt is None else dis_fmt)
@@ -131,18 +134,26 @@ def make_source(cfg: Config, dis_fmt=None, dis_matrix=None, dis_full_range=None,
     if dis_p016_deep is None:
         dis_p016_deep = bool(cfg.flags & _lib.FLAG_P016_DEEP) and src.format in YUV16_FORMATS
     src.flags = _lib.FLAG_P016_DEEP if dis_p016_deep else 0
+    src.width = int(dis_width or 0)
+    src.height = int(dis_height or 0)
     return src
 
 
 def is_mixed(cfg: Config, src: Optional[Source]) -> bool:
-    """Whether ssimu2_create_mixed(cfg, src) makes a mixed handle: the sides differ in format or deep flag, or (NV12 / P016) in
-    matrix or range.  Otherwise the handle is an ordinary one."""
+    """Whether ssimu2_create_mixed(cfg, src) makes a mixed handle: the sides differ in format or deep flag, (YUV) in matrix or
+    range, or in size (a scaled handle).  Otherwise the handle is an ordinary one."""
     if src is None:
         return False
     deep = _lib.FLAG_P016_DEEP
     yuv = cfg.format in YUV_FORMATS
     return not (src.format == cfg.format and (src.flags & deep) == (cfg.flags & deep) and
-                (not yuv or (src.matrix == cfg.matrix and bool(src.full_range) == bool(cfg.full_range))))
+                (not yuv or (src.matrix == cfg.matrix and bool(src.full_range) == bool(cfg.full_range))) and
+                not is_scaled(cfg, src))
+
+
+def is_scaled(cfg: Config, src: Optional[Source]) -> bool:
+    """Whether the distorted frames `src` describes are smaller than the reference frames (upscaled before scoring)."""
+    return src is not None and (src.width or cfg.width, src.height or cfg.height) != (cfg.width, cfg.height)
 
 
 class Ssimulacra2:
@@ -153,7 +164,7 @@ class Ssimulacra2:
                  batch: int = 0, ring: int = 0, pipeline: Optional[str] = None, score_only: bool = False,
                  input_group: int = 0, timing: bool = True, p016_deep: bool = False, dis_fmt: Optional[PixelFormat] = None,
                  dis_matrix: Optional[ColorMatrix] = None, dis_full_range: Optional[bool] = None,
-                 dis_p016_deep: Optional[bool] = None):
+                 dis_p016_deep: Optional[bool] = None, dis_width: Optional[int] = None, dis_height: Optional[int] = None):
         """pipeline: None / "hv" = the product pipeline (front-end, fused H+V kernel, finalize); "split" = development
         pipeline with the H-pass planes in HBM (debug_read(what=1)).
         score_only: SSIMU2_FLAG_SCORE_ONLY -- skip the work whose weights are zero (scores identical, no norms).
@@ -162,7 +173,10 @@ class Ssimulacra2:
         a front-end without the 10-bit memo tables (of the reference frames when the distorted frames are described apart).
         dis_fmt, dis_matrix, dis_full_range, dis_p016_deep: the distorted frames' own description (None = as the reference);
         any of them set creates the handle with ssimu2_create_mixed.  Host frames of a mixed handle are copied with each
-        side's own `nbytes`."""
+        side's own `nbytes`.
+        dis_width, dis_height: the distorted frames' size when it is smaller than width x height (e.g. a 720p encode scored
+        against its 1080p source): they are upscaled to width x height on the GPU (bicubic Catmull-Rom, ssimu2_source) and
+        scored there.  Distorted frames are then given at their own size."""
         self._h = C.c_void_p()
         if pipeline not in (None, "hv", "split"):
             raise ValueError(f"unknown pipeline {pipeline!r}")
@@ -170,13 +184,15 @@ class Ssimulacra2:
                 (_lib.FLAG_P016_DEEP if p016_deep else 0)
         cfg = make_config(width, height, fmt, matrix, full_range, device, batch, ring,
                           _lib.PIPELINE_SPLIT if pipeline == "split" else _lib.PIPELINE_DEFAULT, flags, input_group)
-        src = make_source(cfg, dis_fmt, dis_matrix, dis_full_range, dis_p016_deep)
+        src = make_source(cfg, dis_fmt, dis_matrix, dis_full_range, dis_p016_deep, dis_width, dis_height)
         if src is None:
             check(_lib.lib().ssimu2_create(C.byref(self._h), C.byref(cfg)), "ssimu2_create")
         else:
             check(_lib.lib().ssimu2_create_mixed(C.byref(self._h), C.byref(cfg), C.byref(src)), "ssimu2_create_mixed")
         self.width, self.height, self.format = width, height, PixelFormat(fmt)
         self.dis_format = self.format if src is None else PixelFormat(src.format)
+        self.dis_width = src.width if src is not None and src.width else width
+        self.dis_height = src.height if src is not None and src.height else height
         self.mixed = is_mixed(cfg, src)
         self._keep = {}
         self._last = None
@@ -375,13 +391,15 @@ class ShardedSsimulacra2:
     def __init__(self, width: int, height: int, fmt: PixelFormat, devices: Sequence[int], matrix: ColorMatrix = ColorMatrix.BT709,
                  full_range: bool = False, batch: int = 0, ring: int = 0, score_only: bool = False,
                  dis_fmt: Optional[PixelFormat] = None, dis_matrix: Optional[ColorMatrix] = None,
-                 dis_full_range: Optional[bool] = None, dis_p016_deep: Optional[bool] = None):
-        """dis_*: the distorted frames' own description, as for `Ssimulacra2` (every worker's handle is ssimu2_create_mixed)."""
+                 dis_full_range: Optional[bool] = None, dis_p016_deep: Optional[bool] = None, dis_width: Optional[int] = None,
+                 dis_height: Optional[int] = None):
+        """dis_*: the distorted frames' own description and size, as for `Ssimulacra2` (every worker's handle is
+        ssimu2_create_mixed)."""
         self._s = C.c_void_p()
         flags = _lib.FLAG_SCORE_ONLY if score_only else 0
         cfg = make_config(width, height, fmt, matrix, full_range, 0, batch, ring, _lib.PIPELINE_DEFAULT, flags, 0)
         devs = (C.c_int32 * len(devices))(*devices)
-        src = make_source(cfg, dis_fmt, dis_matrix, dis_full_range, dis_p016_deep)
+        src = make_source(cfg, dis_fmt, dis_matrix, dis_full_range, dis_p016_deep, dis_width, dis_height)
         if src is None:
             check(_lib.lib().ssimu2_shard_create(C.byref(self._s), C.byref(cfg), devs, len(devices)), "ssimu2_shard_create")
         else:

@@ -202,3 +202,84 @@ def make_pair_linearf32(w: int, h: int, frame: int = 0, seed: int = 1, device="c
         d = _distort(p, g, device, 1.5 / 255.0, 4.0 / 255.0)
         chans_d.append(d * d)
     return torch.stack(chans, dim=-1).contiguous(), torch.stack(chans_d, dim=-1).contiguous()
+
+
+# sample planes of each format (make_pair_scaled): (sample dtype, chroma subsampling or "rgb")
+SCALED_FORMATS = {"NV12": ("u8", "420"), "P016": ("u16", "420"), "NV16": ("u8", "422"), "P216": ("u16", "422"),
+                  "YUV444": ("u8", "444"), "YUV444P16": ("u16", "444"), "SRGB8": ("u8", "rgb"), "SRGB16": ("u16", "rgb"),
+                  "SRGBF32": ("f32", "rgb"), "LINEARF32": ("f32", "rgb")}
+
+
+def _area(p, h, w):
+    """Area-downscale a float plane (H, W) to (h, w) (the identity when the size is unchanged)."""
+    if tuple(p.shape) == (h, w):
+        return p
+    return F.interpolate(p[None, None], size=(h, w), mode="area")[0, 0]
+
+
+def make_pair_scaled(fmt: str, w: int, h: int, dis_w: int, dis_h: int, frame: int = 0, seed: int = 1):
+    """A seeded (reference, lower-resolution distorted) pair of format `fmt` (a SCALED_FORMATS name): the reference content
+    at w x h, the distorted frame its area-downscale to dis_w x dis_h (each plane on its own grid) with the distortion of
+    the other generators applied.  -> (ref_planes, dis_planes): lists of numpy sample arrays, one per plane, with
+    interleaved channels side by side in a row -- YUV 4:2:0 / 4:2:2: [Y (h, w), CbCr (chroma rows, 2 * ceil(w / 2))];
+    4:4:4: [Y, Cb, Cr]; packed RGB: [(h, 3 * w)].  8-bit YUV is limited range, 16-bit YUV 10-bit codes in the high bits."""
+    dt, sub = SCALED_FORMATS[fmt]
+    g = _gen(seed, frame, "cpu")
+    q = 4.0 / 219.0
+    if sub == "rgb":
+        ref, dis = [], []
+        for c in range(3):
+            p = _base_luma(h, w, frame, g, "cpu", phase=0.17 * c)
+            d = _distort(_area(p, dis_h, dis_w), g, "cpu", 1.5 / 255.0, 4.0 / 255.0)
+            ref.append(p)
+            dis.append(d)
+
+        def pack(chans):
+            x = torch.stack(chans, dim=-1)
+            if fmt == "LINEARF32":
+                x = x * x
+            if dt == "f32":
+                x = x.float()
+            else:
+                x = torch.round(x * (255 if dt == "u8" else 65535)).clamp(0, 255 if dt == "u8" else 65535).to(torch.int32)
+            return [x.reshape(x.shape[0], -1).numpy().astype({"u8": "uint8", "u16": "uint16", "f32": "float32"}[dt])]
+        return pack(ref), pack(dis)
+    bits = 8 if dt == "u8" else 16
+
+    def grid(ww, hh):
+        return ((hh + 1) // 2 if sub == "420" else hh), ((ww + 1) // 2 if sub != "444" else ww)
+    ch, cw = grid(w, h)
+    dch, dcw = grid(dis_w, dis_h)
+    lum = _base_luma(h, w, frame, g, "cpu")
+    yy = torch.arange(ch, dtype=torch.float32)[:, None] / max(ch - 1, 1)
+    xx = torch.arange(cw, dtype=torch.float32)[None, :] / max(cw - 1, 1)
+    cb = (0.5 + 0.2 * (xx - 0.5) * 2 * torch.cos(2 * math.pi * (yy + frame / 131.0)) + 0.05 * _smooth_noise(ch, cw, 8, g, "cpu")).clamp(0, 1)
+    cr = (0.5 + 0.2 * (yy - 0.5) * 2 * torch.sin(2 * math.pi * (xx + frame / 171.0)) + 0.05 * _smooth_noise(ch, cw, 8, g, "cpu")).clamp(0, 1)
+    lum_d = _distort(_area(lum, dis_h, dis_w), g, "cpu", 1.5 / 255.0, q)
+    cb_d = _distort(_area(cb, dch, dcw), g, "cpu", 0.75 / 255.0, q)
+    cr_d = _distort(_area(cr, dch, dcw), g, "cpu", 0.75 / 255.0, q)
+    npdt = "uint8" if bits == 8 else "uint16"
+
+    def pack(yv, u, v):
+        yq, uq, vq = (t.numpy().astype(npdt) for t in quantize_yuv(yv, u, v, bits))
+        if sub == "444":
+            return [yq, uq, vq]
+        import numpy as np
+        uv = np.zeros((uq.shape[0], 2 * uq.shape[1]), npdt)
+        uv[:, 0::2], uv[:, 1::2] = uq, vq
+        return [yq, uv]
+    return pack(lum, cb, cr), pack(lum_d, cb_d, cr_d)
+
+
+def compact_planes(planes):
+    """Sample planes (make_pair_scaled's form) -> (buf: 1-D numpy uint8 array, pitch, plane1 offset or 0): the compact layout
+    of a scaled handle's staged frames (pitch = the longest row rounded up to 256 bytes, plane i at i * pitch * h; 4:4:4 Cr at
+    plane[1] + (plane[1] - plane[0]))."""
+    import numpy as np
+    h = planes[0].shape[0]
+    pitch = (max(p.shape[1] * p.itemsize for p in planes) + 255) // 256 * 256
+    buf = np.zeros(pitch * h * len(planes), np.uint8)
+    for i, p in enumerate(planes):
+        rows = np.ascontiguousarray(p).view(np.uint8).reshape(p.shape[0], -1)
+        buf[i * pitch * h: i * pitch * h + p.shape[0] * pitch].reshape(p.shape[0], pitch)[:, :rows.shape[1]] = rows
+    return buf, pitch, (pitch * h if len(planes) > 1 else 0)
