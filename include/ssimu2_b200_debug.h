@@ -18,6 +18,14 @@ extern "C" {
  *           (SSIMU2_PIPELINE_SPLIT only: the default pipeline never materialises these planes)
  * Only valid until that slot is reused (i.e. right after ssimu2_get_score). */
 int ssimu2_debug_read(ssimu2_t *h, uint64_t ticket, int what, int scale, float *out, size_t out_floats);
+/* Copy the per-strip partial sums of the pair `ticket` (same slot rule as ssimu2_debug_read) to host memory:
+ * double[total_strips][3][6], channel x {ssim L1, ssim L4, artifact L1, artifact L4, detail L1, detail L4}, where an
+ * L1 entry is the strip's sum of the map and an L4 entry the sum of its fourth power (k_finalize reduces them to the norms).
+ * The strips of scale s are rows strip0[s] .. strip0[s] + n_strips[s] - 1 (ssimu2_debug_strips); out_doubles >= 18 * total. */
+int ssimu2_debug_read_partials(ssimu2_t *h, uint64_t ticket, double *out, size_t out_doubles);
+/* Strip geometry of the partial-sum table: per scale (nscales of ssimu2_get_info) the first row and the number of strips;
+ * *strip_cols = columns per strip (strip k of a scale covers columns [k * cols, (k + 1) * cols) of that scale). */
+int ssimu2_debug_strips(const ssimu2_t *h, uint32_t strip0[6], uint32_t n_strips[6], uint32_t *strip_cols);
 /* Run the device arithmetic helpers over an array (host pointers) so the tests can compare them bit for
  * bit with libm / IEEE division:  op 0: out[i] = cbrtf(in[i]);  op 1: powf(in[i], y);  op 2: in[i] / y (f32);
  * op 3: `in` holds n (num, den) pairs of DOUBLES, `out` n doubles: num / den;

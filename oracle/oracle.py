@@ -176,6 +176,22 @@ def blur_plane(plane: np.ndarray) -> np.ndarray:
     return blur_vertical(blur_horizontal(plane))
 
 
+def map_inputs(ref_lin: np.ndarray, dis_lin: np.ndarray, scale: int):
+    """Per-pixel inputs of the error maps of one scale (cpu.rs:604-627, :658-662), the f32 values ssim_map and
+    edge_diff_map evaluate their maps from: -> (q, a, b), each float32 (3, H_s, W_s): q = the SSIM' quotient
+    num_m * num_s / denom_s, a = |x2 - mu2|, b = |x1 - mu1|.  None when the pyramid has no such scale."""
+    ref_lin, dis_lin = _f32(ref_lin), _f32(dis_lin)
+    assert ref_lin.shape == dis_lin.shape and ref_lin.shape[0] == 3
+    _, h, w = ref_lin.shape
+    for _ in range(scale):
+        w, h = (w + 1) // 2, (h + 1) // 2
+    q, a, b = (np.empty((3, h, w), np.float32) for _ in range(3))
+    _, h0, w0 = ref_lin.shape
+    if lib().oracle_map_inputs(_p(ref_lin), _p(dis_lin), w0, h0, scale, _p(q), _p(a), _p(b)) != 0:
+        return None
+    return q, a, b
+
+
 # ---------------------------------------------------------------- whole metric
 def ssimu2_linear_planar(ref_lin: np.ndarray, dis_lin: np.ndarray):
     """-> (score, norms[108], nscales).  norms index = c*36 + s*6 + n*3 + m (WEIGHT order)."""

@@ -460,24 +460,36 @@ void oracle_blur_plane(const float *in, float *out, float *temp, int w, int h)
 /* ------------------------------------------------------------------------------------ */
 /* Error maps and their norms.  cpu.rs:581-683.                                          */
 /* ------------------------------------------------------------------------------------ */
+/* The f32 part of both maps at one pixel: the SSIM' quotient num_m * num_s / denom_s (cpu.rs:604-627) and the edge
+ * map's a = |x2 - mu2|, b = |x1 - mu1| (cpu.rs:658-662).  Everything after these three values is f64 in the reference. */
+static inline float ssim_quotient(float mu1, float mu2, float s11, float s22, float s12)
+{
+    const float C2 = 0.0009f;
+    float mu11 = mu1 * mu1, mu22 = mu2 * mu2, mu12 = mu1 * mu2;
+    float mu_diff = mu1 - mu2;
+    float num_m = fmaf(mu_diff, -mu_diff, 1.0f);
+    float num_s = fmaf(2.0f, s12 - mu12, C2);
+    float denom_s = (s11 - mu11) + (s22 - mu22) + C2;
+    return (num_m * num_s) / denom_s;
+}
+
+static inline void edge_inputs(float x1, float mu1, float x2, float mu2, float *a, float *b)
+{
+    *a = fabsf(x2 - mu2);
+    *b = fabsf(x1 - mu1);
+}
+
 /* ssim_map: out6 = {L1,L4} x 3 channels as plane_averages[c*2 + n] */
 static void ssim_map(int w, int h, const float *m1, const float *m2, const float *s11,
                      const float *s22, const float *s12, double out6[6])
 {
-    const float C2 = 0.0009f;
     size_t n = (size_t)w * h;
     double one_per_pixels = 1.0 / (double)n;
     for (int c = 0; c < 3; c++) {
         double sum0 = 0.0, sum1 = 0.0;
         for (size_t i = 0; i < n; i++) {
             size_t k = c * n + i;
-            float mu1 = m1[k], mu2 = m2[k];
-            float mu11 = mu1 * mu1, mu22 = mu2 * mu2, mu12 = mu1 * mu2;
-            float mu_diff = mu1 - mu2;
-            float num_m = fmaf(mu_diff, -mu_diff, 1.0f);
-            float num_s = fmaf(2.0f, s12[k] - mu12, C2);
-            float denom_s = (s11[k] - mu11) + (s22[k] - mu22) + C2;
-            double d = 1.0 - (double)((num_m * num_s) / denom_s);
+            double d = 1.0 - (double)ssim_quotient(m1[k], m2[k], s11[k], s22[k], s12[k]);
             d = d > 0.0 ? d : 0.0; /* f64::max(0.0); NaN -> 0.0 like Rust's max */
             if (d != d) d = 0.0;
             sum0 += d;
@@ -499,7 +511,9 @@ static void edge_diff_map(int w, int h, const float *img1, const float *mu1, con
         double s0 = 0, s1 = 0, s2 = 0, s3 = 0;
         for (size_t i = 0; i < n; i++) {
             size_t k = c * n + i;
-            double d1 = (1.0 + (double)fabsf(img2[k] - mu2[k])) / (1.0 + (double)fabsf(img1[k] - mu1[k])) - 1.0;
+            float a, b;
+            edge_inputs(img1[k], mu1[k], img2[k], mu2[k], &a, &b);
+            double d1 = (1.0 + (double)a) / (1.0 + (double)b) - 1.0;
             double artifact = d1 > 0.0 ? d1 : 0.0;
             s0 += artifact;
             double a2 = artifact * artifact;
@@ -563,6 +577,70 @@ double oracle_score_from_averages(int nscales, const double (*ssim6)[6], const d
     return ssim;
 }
 
+/* The per-scale stages of compute_frame_ssimulacra2 (cpu.rs:342-410): downscale, XYB, the five blurred planes. */
+typedef struct {
+    int w, h; /* size of the current scale */
+    float *img1, *img2, *tmp, *x1, *x2, *mul, *temp, *s11, *s22, *s12, *mu1, *mu2;
+} pyramid_t;
+
+static void pyramid_init(pyramid_t *p, const float *ref_lin, const float *dis_lin, int w0, int h0)
+{
+    size_t n0 = (size_t)w0 * h0;
+    p->w = w0; p->h = h0;
+    p->img1 = malloc(3 * n0 * sizeof(float)); p->img2 = malloc(3 * n0 * sizeof(float));
+    p->tmp = malloc(3 * n0 * sizeof(float));
+    p->x1 = malloc(3 * n0 * sizeof(float)); p->x2 = malloc(3 * n0 * sizeof(float));
+    p->mul = malloc(3 * n0 * sizeof(float)); p->temp = malloc(n0 * sizeof(float));
+    p->s11 = malloc(3 * n0 * sizeof(float)); p->s22 = malloc(3 * n0 * sizeof(float));
+    p->s12 = malloc(3 * n0 * sizeof(float)); p->mu1 = malloc(3 * n0 * sizeof(float));
+    p->mu2 = malloc(3 * n0 * sizeof(float));
+    memcpy(p->img1, ref_lin, 3 * n0 * sizeof(float));
+    memcpy(p->img2, dis_lin, 3 * n0 * sizeof(float));
+}
+
+static void pyramid_free(pyramid_t *p)
+{
+    free(p->img1); free(p->img2); free(p->tmp); free(p->x1); free(p->x2); free(p->mul); free(p->temp);
+    free(p->s11); free(p->s22); free(p->s12); free(p->mu1); free(p->mu2);
+}
+
+/* Move to scale `scale` (called for 0, 1, 2, ... in turn): the downscaled linear images.  Returns 0 when the image of
+ * the previous scale is smaller than 8x8 (cpu.rs:359): that scale and every later one do not exist. */
+static int pyramid_down(pyramid_t *p, int scale)
+{
+    int w = p->w, h = p->h;
+    if (w < 8 || h < 8)
+        return 0;
+    if (scale > 0) {
+        oracle_downscale_by_2(p->img1, w, h, p->tmp);
+        int nw = (w + 1) / 2, nh = (h + 1) / 2;
+        memcpy(p->img1, p->tmp, 3 * (size_t)nw * nh * sizeof(float));
+        oracle_downscale_by_2(p->img2, w, h, p->tmp);
+        memcpy(p->img2, p->tmp, 3 * (size_t)nw * nh * sizeof(float));
+        p->w = nw; p->h = nh;
+    }
+    return 1;
+}
+
+/* XYB and the five blurred planes of the current scale. */
+static void pyramid_planes(pyramid_t *p)
+{
+    int w = p->w, h = p->h;
+    size_t n = (size_t)w * h;
+    oracle_linear_to_xyb(p->img1, w, h, p->x1);
+    oracle_linear_to_xyb(p->img2, w, h, p->x2);
+
+    /* image_multiply + blur, cpu.rs:388-399 */
+    for (size_t i = 0; i < 3 * n; i++) p->mul[i] = p->x1[i] * p->x1[i];
+    for (int c = 0; c < 3; c++) oracle_blur_plane(p->mul + c * n, p->s11 + c * n, p->temp, w, h);
+    for (size_t i = 0; i < 3 * n; i++) p->mul[i] = p->x2[i] * p->x2[i];
+    for (int c = 0; c < 3; c++) oracle_blur_plane(p->mul + c * n, p->s22 + c * n, p->temp, w, h);
+    for (size_t i = 0; i < 3 * n; i++) p->mul[i] = p->x1[i] * p->x2[i];
+    for (int c = 0; c < 3; c++) oracle_blur_plane(p->mul + c * n, p->s12 + c * n, p->temp, w, h);
+    for (int c = 0; c < 3; c++) oracle_blur_plane(p->x1 + c * n, p->mu1 + c * n, p->temp, w, h);
+    for (int c = 0; c < 3; c++) oracle_blur_plane(p->x2 + c * n, p->mu2 + c * n, p->temp, w, h);
+}
+
 /* compute_frame_ssimulacra2, cpu.rs:342-410, on planar linear RGB inputs.
  * norms[108] (optional) receives the per-scale/per-channel averages in WEIGHT order for a
  * full 6-scale run: norms[c*36 + s*6 + n*3 + m], n in {L1,L4}, m in {ssim, artifact, detail};
@@ -571,48 +649,18 @@ double oracle_score_from_averages(int nscales, const double (*ssim6)[6], const d
 int oracle_ssimu2_linear_planar(const float *ref_lin, const float *dis_lin, int w0, int h0,
                                 double *score, double *norms)
 {
-    int w = w0, h = h0;
-    size_t n0 = (size_t)w0 * h0;
-    float *img1 = malloc(3 * n0 * sizeof(float)), *img2 = malloc(3 * n0 * sizeof(float));
-    float *tmp = malloc(3 * n0 * sizeof(float));
-    float *x1 = malloc(3 * n0 * sizeof(float)), *x2 = malloc(3 * n0 * sizeof(float));
-    float *mul = malloc(3 * n0 * sizeof(float)), *temp = malloc(n0 * sizeof(float));
-    float *s11 = malloc(3 * n0 * sizeof(float)), *s22 = malloc(3 * n0 * sizeof(float));
-    float *s12 = malloc(3 * n0 * sizeof(float)), *mu1 = malloc(3 * n0 * sizeof(float));
-    float *mu2 = malloc(3 * n0 * sizeof(float));
+    pyramid_t p;
     double ssim6[NUM_SCALES][6], edge12[NUM_SCALES][12];
     int nscales = 0;
-    memcpy(img1, ref_lin, 3 * n0 * sizeof(float));
-    memcpy(img2, dis_lin, 3 * n0 * sizeof(float));
+    pyramid_init(&p, ref_lin, dis_lin, w0, h0);
     if (norms) memset(norms, 0, 108 * sizeof(double));
 
     for (int scale = 0; scale < NUM_SCALES; scale++) {
-        if (w < 8 || h < 8)
+        if (!pyramid_down(&p, scale))
             break;
-        if (scale > 0) {
-            oracle_downscale_by_2(img1, w, h, tmp);
-            int nw = (w + 1) / 2, nh = (h + 1) / 2;
-            memcpy(img1, tmp, 3 * (size_t)nw * nh * sizeof(float));
-            oracle_downscale_by_2(img2, w, h, tmp);
-            memcpy(img2, tmp, 3 * (size_t)nw * nh * sizeof(float));
-            w = nw; h = nh;
-        }
-        size_t n = (size_t)w * h;
-        oracle_linear_to_xyb(img1, w, h, x1);
-        oracle_linear_to_xyb(img2, w, h, x2);
-
-        /* image_multiply + blur, cpu.rs:388-399 */
-        for (size_t i = 0; i < 3 * n; i++) mul[i] = x1[i] * x1[i];
-        for (int c = 0; c < 3; c++) oracle_blur_plane(mul + c * n, s11 + c * n, temp, w, h);
-        for (size_t i = 0; i < 3 * n; i++) mul[i] = x2[i] * x2[i];
-        for (int c = 0; c < 3; c++) oracle_blur_plane(mul + c * n, s22 + c * n, temp, w, h);
-        for (size_t i = 0; i < 3 * n; i++) mul[i] = x1[i] * x2[i];
-        for (int c = 0; c < 3; c++) oracle_blur_plane(mul + c * n, s12 + c * n, temp, w, h);
-        for (int c = 0; c < 3; c++) oracle_blur_plane(x1 + c * n, mu1 + c * n, temp, w, h);
-        for (int c = 0; c < 3; c++) oracle_blur_plane(x2 + c * n, mu2 + c * n, temp, w, h);
-
-        ssim_map(w, h, mu1, mu2, s11, s22, s12, ssim6[scale]);
-        edge_diff_map(w, h, x1, mu1, x2, mu2, edge12[scale]);
+        pyramid_planes(&p);
+        ssim_map(p.w, p.h, p.mu1, p.mu2, p.s11, p.s22, p.s12, ssim6[scale]);
+        edge_diff_map(p.w, p.h, p.x1, p.mu1, p.x2, p.mu2, edge12[scale]);
         if (norms)
             for (int c = 0; c < 3; c++)
                 for (int nn = 0; nn < 2; nn++) {
@@ -624,9 +672,30 @@ int oracle_ssimu2_linear_planar(const float *ref_lin, const float *dis_lin, int 
     }
     if (score)
         *score = oracle_score_from_averages(nscales, ssim6, edge12);
-    free(img1); free(img2); free(tmp); free(x1); free(x2); free(mul); free(temp);
-    free(s11); free(s22); free(s12); free(mu1); free(mu2);
+    pyramid_free(&p);
     return nscales;
+}
+
+/* The per-pixel inputs of the error maps of one scale, as ssim_map and edge_diff_map see them: q = the SSIM' quotient,
+ * a = |x2 - mu2|, b = |x1 - mu1|, each float[3][h_s][w_s] for the w_s x h_s image of that scale.  From these the maps
+ * are d = max(1 - q, 0) and d1 = (1 + a) / (1 + b) - 1 in f64.  Returns 0, or -1 when the scale does not exist. */
+int oracle_map_inputs(const float *ref_lin, const float *dis_lin, int w0, int h0, int scale, float *q, float *a, float *b)
+{
+    pyramid_t p;
+    int ok = scale >= 0 && scale < NUM_SCALES;
+    pyramid_init(&p, ref_lin, dis_lin, w0, h0);
+    for (int s = 0; ok && s <= scale; s++)
+        ok = pyramid_down(&p, s);
+    if (ok) {
+        pyramid_planes(&p);
+        size_t n = (size_t)p.w * p.h;
+        for (size_t k = 0; k < 3 * n; k++) {
+            q[k] = ssim_quotient(p.mu1[k], p.mu2[k], p.s11[k], p.s22[k], p.s12[k]);
+            edge_inputs(p.x1[k], p.mu1[k], p.x2[k], p.mu2[k], &a[k], &b[k]);
+        }
+    }
+    pyramid_free(&p);
+    return ok ? 0 : -1;
 }
 
 /* Front-end + metric in one call, one per input format of the boundary

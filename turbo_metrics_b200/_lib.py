@@ -89,7 +89,9 @@ SYMBOLS = {
     "ssimu2_scores_device": (C.c_int, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "ssimu2_get_info": (C.c_int, [_P, C.POINTER(Info)]),
     "ssimu2_debug_read": (C.c_int, [_P, C.c_uint64, C.c_int, C.c_int, C.POINTER(C.c_float), C.c_size_t]),
-    "ssimu2_debug_math": (C.c_int, [C.c_int, C.POINTER(C.c_float), C.c_float, C.POINTER(C.c_float), C.c_size_t]),
+    "ssimu2_debug_read_partials": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_double), C.c_size_t]),
+    "ssimu2_debug_strips": (C.c_int, [_P, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+    "ssimu2_debug_math":(C.c_int, [C.c_int, C.POINTER(C.c_float), C.c_float, C.POINTER(C.c_float), C.c_size_t]),
     "ssimu2_last_batch_ms": (C.c_int, [_P, C.POINTER(C.c_float)]),
     "ssimu2_kernel_ms": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int]),
     "ssimu2_shard_create": (C.c_int, [C.POINTER(_P), C.POINTER(Config), C.POINTER(C.c_int32), C.c_uint32]),

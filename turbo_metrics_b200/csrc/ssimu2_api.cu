@@ -1187,18 +1187,28 @@ int ssimu2_get_info(const ssimu2_t* h, ssimu2_info* info)
 }
 
 // ---- include/ssimu2_b200_debug.h ---------------------------------------------------------------
+// The batch slot that served `ticket` and the ticket's frame index in it (valid until the slot is reused).
+static int debug_slot(ssimu2_t* h, uint64_t ticket, Slot** sl, size_t* idx)
+{
+    int si = h->res_slot[ticket % kResultCap];
+    if (si < 0) return SSIMU2_E_TICKET;
+    *sl = &h->slots[si];
+    if (ticket < (*sl)->first_ticket) return SSIMU2_E_TICKET;
+    *idx = (size_t)(ticket - (*sl)->first_ticket);
+    if (*idx >= h->batch) return SSIMU2_E_TICKET;
+    return SSIMU2_OK;
+}
+
 int ssimu2_debug_read(ssimu2_t* h, uint64_t ticket, int what, int scale, float* out, size_t out_floats)
 {
     if (!h || !out || scale < 0 || scale >= h->geo.nscales) return SSIMU2_E_INVALID;
     int r = ssimu2_wait(h, ticket);
     if (r) return r;
     DeviceGuard guard(h->cfg.device);
-    int si = h->res_slot[ticket % kResultCap];
-    if (si < 0) return SSIMU2_E_TICKET;
-    Slot& sl = h->slots[si];
-    if (ticket < sl.first_ticket) return SSIMU2_E_TICKET;
-    size_t idx = (size_t)(ticket - sl.first_ticket);
-    if (idx >= h->batch) return SSIMU2_E_TICKET;
+    Slot* slp;
+    size_t idx;
+    if ((r = debug_slot(h, ticket, &slp, &idx))) return r;
+    Slot& sl = *slp;
     const ScaleDesc& sd = h->geo.sc[scale];
     int planes;
     const float* src;
@@ -1215,6 +1225,33 @@ int ssimu2_debug_read(ssimu2_t* h, uint64_t ticket, int what, int scale, float* 
     if (out_floats < (size_t)planes * sd.w * sd.h) return SSIMU2_E_INVALID;
     CU_TRY(cudaMemcpy2D(out, (size_t)sd.w * sizeof(float), src, (size_t)sd.pitch * sizeof(float),
                         (size_t)sd.w * sizeof(float), (size_t)planes * sd.h, cudaMemcpyDeviceToHost));
+    return SSIMU2_OK;
+}
+
+int ssimu2_debug_read_partials(ssimu2_t* h, uint64_t ticket, double* out, size_t out_doubles)
+{
+    if (!h || !out) return SSIMU2_E_INVALID;
+    int r = ssimu2_wait(h, ticket);
+    if (r) return r;
+    DeviceGuard guard(h->cfg.device);
+    Slot* sl;
+    size_t idx;
+    if ((r = debug_slot(h, ticket, &sl, &idx))) return r;
+    const size_t n = (size_t)h->geo.total_strips * 18;
+    if (out_doubles < n) return SSIMU2_E_INVALID;
+    CU_TRY(cudaMemcpy(out, sl->partials + idx * n, n * sizeof(double), cudaMemcpyDeviceToHost));
+    return SSIMU2_OK;
+}
+
+int ssimu2_debug_strips(const ssimu2_t* h, uint32_t strip0[6], uint32_t n_strips[6], uint32_t* strip_cols)
+{
+    if (!h || !strip0 || !n_strips || !strip_cols) return SSIMU2_E_INVALID;
+    for (int s = 0; s < kMaxScales; s++) {
+        const bool on = s < h->geo.nscales;
+        strip0[s] = on ? (uint32_t)h->geo.sc[s].strip0 : 0u;
+        n_strips[s] = on ? (uint32_t)h->geo.sc[s].n_strips : 0u;
+    }
+    *strip_cols = (uint32_t)kVCols;
     return SSIMU2_OK;
 }
 

@@ -370,6 +370,24 @@ class Ssimulacra2:
                                            out.size), "ssimu2_debug_read")
         return out
 
+    def debug_strips(self):
+        """-> (strip0[nscales], n_strips[nscales], strip_cols): the rows of each scale in the partial-sum table and the
+        columns one strip covers."""
+        s0, ns, cols = (C.c_uint32 * 6)(), (C.c_uint32 * 6)(), C.c_uint32()
+        check(_lib.lib().ssimu2_debug_strips(self._h, s0, ns, C.byref(cols)), "ssimu2_debug_strips")
+        n = self.info().nscales
+        return list(s0)[:n], list(ns)[:n], cols.value
+
+    def debug_partials(self, ticket: int) -> list:
+        """The pair's per-strip partial sums, one float64 array of shape (n_strips, 3, 6) per scale: channel x {ssim L1,
+        ssim L4, artifact L1, artifact L4, detail L1, detail L4} (L1: the strip's sum of the map, L4: of its fourth power).
+        Valid until the batch slot that served the ticket is reused, like debug_read."""
+        strip0, n_strips, _ = self.debug_strips()
+        out = np.zeros((sum(n_strips), 3, 6), np.float64)
+        check(_lib.lib().ssimu2_debug_read_partials(self._h, ticket, out.ctypes.data_as(C.POINTER(C.c_double)), out.size),
+              "ssimu2_debug_read_partials")
+        return [out[s0:s0 + n] for s0, n in zip(strip0, n_strips)]
+
     def kernel_ms(self, reset: bool = False):
         """-> (ms_total[4] for frontend/hpass/vpass/finalize, batches, pairs) since the last reset."""
         ms = (C.c_double * 4)()
