@@ -146,8 +146,28 @@ typedef struct {
     uint32_t pipeline;    /* ssimu2_pipeline */
     uint32_t flags;       /* SSIMU2_FLAG_* */
     uint32_t input_group; /* pairs per front-end launch; 0 = whole batch.  Smaller groups consume the input frames sooner */
-    uint32_t reserved[5]; /* must be 0 */
+    uint32_t tile;        /* tile scores (see below); 0 = off */
+    uint32_t reserved[4]; /* must be 0 */
 } ssimu2_config;
+
+/* Tile scores (ssimu2_config.tile, since ABI 2.3; ssimu2_version() is unchanged, so probe the capability by creating a handle:
+ * an older library returns SSIMU2_E_INVALID for the word).  Besides its frame score, every pair gets a coarse map: one
+ * SSIMULACRA2 score per tile of a grid, for finding WHERE a frame is bad.
+ *   - tile = T, a power of two with 64 <= T <= 32768 (otherwise SSIMU2_E_UNSUPPORTED, as is any T with SSIMU2_PIPELINE_SPLIT;
+ *     both checked before any device call; ssimu2_shard_create / _create_mixed refuse any T != 0).  Tile (ty, tx) covers
+ *     the pixels [tx T, (tx + 1) T) x [ty T, (ty + 1) T), clipped to the frame: tiles_x = ceil(width / T) by
+ *     tiles_y = ceil(height / T) tiles.
+ *   - The pyramid nests exactly: scale-s pixel i is the box of scale-0 pixels [i 2^s, (i + 1) 2^s).  At scale s a tile's
+ *     footprint is the T_s = T >> s square at (tx T_s, ty T_s), clipped to that scale's size; it is never empty.
+ *   - The maps are those of the frame score, computed over the whole frame; only the pooling is restricted.  Per tile, scale
+ *     s, channel c and map m: L1 = sum over the footprint of the map / N_s and L4 = (sum of map^4 / N_s)^(1/4), N_s the
+ *     footprint's pixel count.  These 108 norms (WEIGHT order, see ssimu2_get_norms) give the score exactly as the frame's
+ *     norms give the frame score: the dense weight cursor over the scales that exist, x 0.9562..., the cubic, and
+ *     100 - 10 s^0.6276... (s <= 0 gives 100).
+ *   - So a tile score is NOT the score of the cropped tile (a crop would zero-pad the filters at its edges), the frame score
+ *     is NOT the mean of the tile scores, and a tile whose reference and distorted neighbourhoods are identical scores
+ *     exactly 100.  Frame scores and norms are bit-identical to those of the same handle without tiles, and tile scores are
+ *     bit-identical between the full and the score-only mode. */
 
 /* The description of the DISTORTED frames of a mixed handle (ssimu2_create_mixed); ssimu2_config describes the reference. */
 typedef struct {
@@ -247,6 +267,15 @@ int ssimu2_submit_host_batch(ssimu2_t *h, uint32_t n, const ssimu2_frame *refs, 
  * two sides have different bytes per pixel. */
 int ssimu2_submit_host_sized(ssimu2_t *h, uint32_t n, const ssimu2_frame *refs, size_t ref_bytes, const ssimu2_frame *diss,
                              size_t dis_bytes, uint64_t *first_ticket);
+
+/* ---- tile scores (ssimu2_config.tile) ------------------------------------------------------ */
+/* The handle's tile grid: *tile = ssimu2_config.tile (0: a handle without tiles, the rest 0 too), tiles_x x tiles_y tiles, and
+ * *capacity = how many of the most recent tickets still have their map on the host (at least batch x ring). */
+int ssimu2_get_tile_grid(const ssimu2_t *h, uint32_t *tile, uint32_t *tiles_x, uint32_t *tiles_y, uint64_t *capacity);
+/* The tile scores of a ticket: tiles_y x tiles_x doubles, row-major (flushes and waits like ssimu2_get_score).
+ * SSIMU2_E_UNSUPPORTED on a handle without tiles, SSIMU2_E_INVALID if n is smaller than tiles_x x tiles_y, SSIMU2_E_TICKET
+ * for a ticket not submitted yet or older than the capacity. */
+int ssimu2_get_tile_scores(ssimu2_t *h, uint64_t ticket, double *out, size_t n);
 
 /* ---- results on the device ----------------------------------------------------------- */
 /* Device address of the f64 score ring (one entry per ticket, index ticket % capacity). */

@@ -26,6 +26,13 @@ int ssimu2_debug_read_partials(ssimu2_t *h, uint64_t ticket, double *out, size_t
 /* Strip geometry of the partial-sum table: per scale (nscales of ssimu2_get_info) the first row and the number of strips;
  * *strip_cols = columns per strip (strip k of a scale covers columns [k * cols, (k + 1) * cols) of that scale). */
 int ssimu2_debug_strips(const ssimu2_t *h, uint32_t strip0[6], uint32_t n_strips[6], uint32_t *strip_cols);
+/* The per-tile sums of the pair `ticket` of a tile handle (same slot rule as ssimu2_debug_read): double[entries][3][6] laid out
+ * as ssimu2_debug_read_partials' rows, one entry per (scale, tile row, column unit).  A column unit of scale s is unit_cols[s]
+ * = min(64, T >> s) columns: one tile column, or one 64-column strip of it.  Scale s holds tiles_y x units[s] entries from
+ * entry0[s] on, row-major; out_doubles >= 18 x (the entries of all scales).  SSIMU2_E_UNSUPPORTED on a handle without tiles. */
+int ssimu2_debug_read_tile_partials(ssimu2_t *h, uint64_t ticket, double *out, size_t out_doubles);
+/* Layout of that table per scale (nscales of ssimu2_get_info; 0 beyond). */
+int ssimu2_debug_tile_units(const ssimu2_t *h, uint32_t entry0[6], uint32_t units[6], uint32_t unit_cols[6]);
 /* Run the device arithmetic helpers over an array (host pointers) so the tests can compare them bit for
  * bit with libm / IEEE division:  op 0: out[i] = cbrtf(in[i]);  op 1: powf(in[i], y);  op 2: in[i] / y (f32);
  * op 3: `in` holds n (num, den) pairs of DOUBLES, `out` n doubles: num / den;

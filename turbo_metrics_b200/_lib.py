@@ -19,11 +19,20 @@ class Frame(C.Structure):
 
 
 class Config(C.Structure):
-    """ssimu2_config"""
+    """ssimu2_config.  `tile` (the tile size of the per-tile scores, 0 = off) is the C struct's first of the five words
+    `reserved` views."""
     _fields_ = [("width", C.c_uint32), ("height", C.c_uint32), ("format", C.c_int32),
                 ("matrix", C.c_int32), ("full_range", C.c_int32), ("device", C.c_int32),
                 ("batch", C.c_uint32), ("ring", C.c_uint32), ("pipeline", C.c_uint32), ("flags", C.c_uint32),
                 ("input_group", C.c_uint32), ("reserved", C.c_uint32 * 5)]
+
+    @property
+    def tile(self) -> int:
+        return self.reserved[0]
+
+    @tile.setter
+    def tile(self, v: int):
+        self.reserved[0] = v
 
 
 class Source(C.Structure):
@@ -86,11 +95,16 @@ SYMBOLS = {
     "ssimu2_submit_host": (C.c_int, [_P, _FP, _FP, C.c_size_t, C.POINTER(C.c_uint64)]),
     "ssimu2_submit_host_batch": (C.c_int, [_P, C.c_uint32, _FP, _FP, C.c_size_t, C.POINTER(C.c_uint64)]),
     "ssimu2_submit_host_sized": (C.c_int, [_P, C.c_uint32, _FP, C.c_size_t, _FP, C.c_size_t, C.POINTER(C.c_uint64)]),
+    "ssimu2_get_tile_grid": (C.c_int, [_P, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32),
+                                       C.POINTER(C.c_uint64)]),
+    "ssimu2_get_tile_scores": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_double), C.c_size_t]),
     "ssimu2_scores_device": (C.c_int, [_P, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "ssimu2_get_info": (C.c_int, [_P, C.POINTER(Info)]),
     "ssimu2_debug_read": (C.c_int, [_P, C.c_uint64, C.c_int, C.c_int, C.POINTER(C.c_float), C.c_size_t]),
     "ssimu2_debug_read_partials": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_double), C.c_size_t]),
     "ssimu2_debug_strips": (C.c_int, [_P, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+    "ssimu2_debug_read_tile_partials": (C.c_int, [_P, C.c_uint64, C.POINTER(C.c_double), C.c_size_t]),
+    "ssimu2_debug_tile_units": (C.c_int, [_P, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
     "ssimu2_debug_math":(C.c_int, [C.c_int, C.POINTER(C.c_float), C.c_float, C.POINTER(C.c_float), C.c_size_t]),
     "ssimu2_last_batch_ms": (C.c_int, [_P, C.POINTER(C.c_float)]),
     "ssimu2_kernel_ms": (C.c_int, [_P, C.POINTER(C.c_double), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int]),

@@ -68,6 +68,9 @@ struct Slot {
     double* scores_d = nullptr;       // [batch]
     double* norms_h = nullptr;        // pinned
     double* scores_h = nullptr;       // pinned
+    double* tiles = nullptr;          // tile handle: k_hv<true>'s tile table [batch][tile_entries][18]
+    double* tile_scores_d = nullptr;  // [batch][tiles_y][tiles_x]
+    double* tile_scores_h = nullptr;  // pinned
     uint8_t* staging = nullptr;       // device staging for host frames: [batch][2][staging_frame_bytes]
     FramePair* in_h = nullptr;        // pinned frame table of the batch being recorded
     FramePair* in_d = nullptr;        // its device copy (uploaded per front-end launch)
@@ -127,6 +130,12 @@ struct ssimu2_handle {
     uint64_t timed_batches = 0, timed_pairs = 0;
     uint64_t alg_bytes = 0, io_bytes = 0;
     unsigned char lite[kMaxScales] = {};   // score-only: channels without SSIM' per scale (HvArgs::lite)
+    // tile scores (ssimu2_config.tile != 0): grid, entries of a frame's tile table, and the host ring of the last tile_cap maps
+    uint32_t tile = 0, tiles_x = 0, tiles_y = 0;
+    int tile_log2 = 0;
+    size_t tile_entries = 0;
+    uint64_t tile_cap = 0;
+    std::vector<double> res_tiles;    // [tile_cap][tiles_y * tiles_x]
 };
 
 namespace {
@@ -586,12 +595,18 @@ static int launch_batch(ssimu2_handle* h, int si)
         a.nframes = (int)n;
         a.lite_bits = 0;
         for (int s = 0; s < kMaxScales; s++) a.lite_bits |= (uint32_t)(h->lite[s] & 7u) << (4 * s);
+        a.tiles = sl.tiles;
+        a.tile_log2 = h->tile_log2;
         if (timed) cudaEventRecord(sl.ev_k[2], st);
-        k_hv<<<(unsigned)(g.items_v * n), kXThreads, kXSmemBytes, st>>>(g, sl.maps_x, a);
+        if (h->tile)
+            k_hv<true><<<(unsigned)(g.items_v * n), kXThreads, kXSmemBytes, st>>>(g, sl.maps_x, a);
+        else
+            k_hv<false><<<(unsigned)(g.items_v * n), kXThreads, kXSmemBytes, st>>>(g, sl.maps_x, a);
         if (timed) cudaEventRecord(sl.ev_k[3], st);
         k_finalize<<<n, 128, 0, st>>>(g, sl.partials, sl.norms_d, h->scores_ring_d, sl.first_ticket, kResultCap, sl.scores_d, a.ticket);
+        if (h->tile) k_tile_finalize<<<dim3(h->tiles_x * h->tiles_y, n), 128, 0, st>>>(g, sl.tiles, h->tile_log2, sl.tile_scores_d);
         if (timed) cudaEventRecord(sl.ev_k[4], st);
-        h->launches += 2;
+        h->launches += h->tile ? 3 : 2;
     } else {
         k_hpass<<<dim3(g.items_h, n), kHThreads, kHSmemBytes, st>>>(g, sl.maps_h);
         if (timed) cudaEventRecord(sl.ev_k[2], st);
@@ -605,6 +620,9 @@ static int launch_batch(ssimu2_handle* h, int si)
     CU_TRY(cudaMemcpyAsync(sl.scores_h, sl.scores_d, n * sizeof(double), cudaMemcpyDeviceToHost, st));
     if (!h->score_only)
         CU_TRY(cudaMemcpyAsync(sl.norms_h, sl.norms_d, (size_t)n * 108 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (h->tile)
+        CU_TRY(cudaMemcpyAsync(sl.tile_scores_h, sl.tile_scores_d, (size_t)n * h->tiles_x * h->tiles_y * sizeof(double),
+                               cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaEventRecord(sl.ev_done, st));
     sl.inflight = true;
     sl.was_timed = timed;
@@ -622,6 +640,10 @@ static int harvest(ssimu2_handle* h, uint32_t si)
         h->res_scores[r] = sl.scores_h[i];
         if (!h->score_only) memcpy(&h->res_norms[r * 108], &sl.norms_h[(size_t)i * 108], 108 * sizeof(double));
         h->res_slot[r] = (int32_t)si;
+        if (h->tile) {
+            const size_t nt = (size_t)h->tiles_x * h->tiles_y;
+            memcpy(&h->res_tiles[(t % h->tile_cap) * nt], &sl.tile_scores_h[i * nt], nt * sizeof(double));
+        }
     }
     if (sl.was_timed) {
         // fused: front-end [0,1], k_hv [2,3], (no separate V pass), finalize [3,4]; split: front-end [0,1], H [1,2], V [2,3], finalize [3,4]
@@ -796,8 +818,11 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
     if (cfg->flags & ~(SSIMU2_FLAG_SCORE_ONLY | SSIMU2_FLAG_NO_TIMING | SSIMU2_FLAG_P016_DEEP)) return SSIMU2_E_UNSUPPORTED;
     if ((cfg->flags & SSIMU2_FLAG_P016_DEEP) && !format_is_yuv16(cfg->format)) return SSIMU2_E_UNSUPPORTED;
     if ((cfg->flags & SSIMU2_FLAG_SCORE_ONLY) && cfg->pipeline != SSIMU2_PIPELINE_DEFAULT) return SSIMU2_E_UNSUPPORTED;
-    for (int i = 0; i < 5; i++)
+    for (int i = 0; i < 4; i++)
         if (cfg->reserved[i]) return SSIMU2_E_INVALID;
+    if (cfg->tile && (cfg->tile < 64 || cfg->tile > 32768 || (cfg->tile & (cfg->tile - 1)) ||
+                      cfg->pipeline != SSIMU2_PIPELINE_DEFAULT))
+        return SSIMU2_E_UNSUPPORTED;
     if (dis) {
         const int rc = check_source(cfg, dis);
         if (rc) return rc;
@@ -859,6 +884,18 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
                 if (w108[base + 0] == 0.0 && w108[base + 3] == 0.0) h->lite[s] |= (unsigned char)(1u << c);
             }
     }
+    if (cfg->tile) {
+        h->tile = cfg->tile;
+        while ((1u << h->tile_log2) < cfg->tile) h->tile_log2++;
+        h->tiles_x = (cfg->width + cfg->tile - 1) / cfg->tile;
+        h->tiles_y = (cfg->height + cfg->tile - 1) / cfg->tile;
+        int none;
+        h->tile_entries = (size_t)tile_layout(h->geo, h->tile_log2, h->geo.nscales, &none);
+        // the host keeps the maps of the last tile_cap tickets (at least four rings' worth of batches), at most ~256 MiB of them
+        const uint64_t map_bytes = (uint64_t)h->tiles_x * h->tiles_y * sizeof(double);
+        const uint64_t want = std::max<uint64_t>(1024, 4ull * h->batch * h->ring);
+        h->tile_cap = std::max<uint64_t>((uint64_t)h->batch * h->ring, std::min<uint64_t>(want, (256ull << 20) / map_bytes));
+    }
     DeviceGuard guard(cfg->device);
     int rc = 0;
 #define CR(expr)                                  \
@@ -875,6 +912,7 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
         h->res_scores.assign(kResultCap, 0.0);
         h->res_norms.assign(kResultCap * 108, 0.0);
         h->res_slot.assign(kResultCap, -1);
+        h->res_tiles.assign((size_t)h->tile_cap * h->tiles_x * h->tiles_y, 0.0);
         for (auto& sl : h->slots) sl.fe_seq.assign(h->batch, 0);
     } catch (...) {
         rc = SSIMU2_E_NOMEM;
@@ -885,7 +923,8 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
     h->device_bytes += kResultCap * sizeof(double);
     CR(cudaFuncSetAttribute((const void*)k_hpass, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kHSmemBytes));
     CR(cudaFuncSetAttribute((const void*)k_vpass, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kVSmemBytes));
-    CR(cudaFuncSetAttribute((const void*)k_hv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kXSmemBytes));
+    CR(cudaFuncSetAttribute((const void*)k_hv<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kXSmemBytes));
+    if (h->tile) CR(cudaFuncSetAttribute((const void*)k_hv<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kXSmemBytes));
     {
         exact_math::CbrtScale cs;
         for (int i = 0; i < 256; i++) cs.tab[i] = exact_math::cbrt_scale_entry(i);
@@ -939,6 +978,17 @@ int ssimu2_create_mixed(ssimu2_t** out, const ssimu2_config* cfg, const ssimu2_s
         CR(cudaMallocHost(&sl.norms_h, (size_t)h->batch * 108 * sizeof(double)));
         CR(cudaMallocHost(&sl.scores_h, (size_t)h->batch * sizeof(double)));
         h->device_bytes += xyb_b + hb_b + hs_b + fl_b + part_b + in_b + (size_t)h->batch * 109 * sizeof(double);
+        if (h->tile) {
+            // every entry k_hv<true> owns is rewritten per batch; the SSIM' entries of X and B of a score-only handle's lite
+            // strips are never written and stay 0
+            const size_t tab_b = h->tile_entries * 18 * h->batch * sizeof(double);
+            const size_t ts_b = (size_t)h->tiles_x * h->tiles_y * h->batch * sizeof(double);
+            CR(cudaMalloc(&sl.tiles, tab_b));
+            CR(cudaMemset(sl.tiles, 0, tab_b));
+            CR(cudaMalloc(&sl.tile_scores_d, ts_b));
+            CR(cudaMallocHost(&sl.tile_scores_h, ts_b));
+            h->device_bytes += tab_b + ts_b;
+        }
         if (h->scaled) {
             const size_t rs_b = (size_t)h->rs_group * h->rs.dst_stride;
             CR(cudaMalloc(&sl.rs_frames, rs_b));
@@ -972,7 +1022,8 @@ int ssimu2_destroy(ssimu2_t* h)
         for (cudaEvent_t e : sl.ev_fe) cudaEventDestroy(e);
         cudaFree(sl.xyb); cudaFree(sl.hb); cudaFree(sl.hstate); cudaFree(sl.hvflags); cudaFree(sl.partials);
         cudaFree(sl.norms_d); cudaFree(sl.scores_d); cudaFree(sl.staging); cudaFree(sl.in_d);
-        cudaFree(sl.rs_frames); cudaFree(sl.rs_in_d);
+        cudaFree(sl.rs_frames); cudaFree(sl.rs_in_d); cudaFree(sl.tiles); cudaFree(sl.tile_scores_d);
+        if (sl.tile_scores_h) cudaFreeHost(sl.tile_scores_h);
         if (sl.in_h) cudaFreeHost(sl.in_h);
         if (sl.rs_in_h) cudaFreeHost(sl.rs_in_h);
         if (sl.norms_h) cudaFreeHost(sl.norms_h);
@@ -1156,6 +1207,29 @@ int ssimu2_stream_wait_input(ssimu2_t* h, uint64_t ticket, void* stream)
     return SSIMU2_OK;
 }
 
+int ssimu2_get_tile_grid(const ssimu2_t* h, uint32_t* tile, uint32_t* tiles_x, uint32_t* tiles_y, uint64_t* capacity)
+{
+    if (!h || !tile || !tiles_x || !tiles_y || !capacity) return SSIMU2_E_INVALID;
+    *tile = h->tile;
+    *tiles_x = h->tiles_x;
+    *tiles_y = h->tiles_y;
+    *capacity = h->tile_cap;
+    return SSIMU2_OK;
+}
+
+int ssimu2_get_tile_scores(ssimu2_t* h, uint64_t ticket, double* out, size_t n)
+{
+    if (!h || !out) return SSIMU2_E_INVALID;
+    if (!h->tile) return SSIMU2_E_UNSUPPORTED;
+    const size_t nt = (size_t)h->tiles_x * h->tiles_y;
+    if (n < nt) return SSIMU2_E_INVALID;
+    if (ticket >= h->next_ticket || h->next_ticket - ticket > h->tile_cap) return SSIMU2_E_TICKET;
+    int r = ssimu2_wait(h, ticket);
+    if (r) return r;
+    memcpy(out, &h->res_tiles[(ticket % h->tile_cap) * nt], nt * sizeof(double));
+    return SSIMU2_OK;
+}
+
 int ssimu2_scores_device(ssimu2_t* h, uint64_t* dptr, uint64_t* capacity)
 {
     if (!h || !dptr || !capacity) return SSIMU2_E_INVALID;
@@ -1252,6 +1326,36 @@ int ssimu2_debug_strips(const ssimu2_t* h, uint32_t strip0[6], uint32_t n_strips
         n_strips[s] = on ? (uint32_t)h->geo.sc[s].n_strips : 0u;
     }
     *strip_cols = (uint32_t)kVCols;
+    return SSIMU2_OK;
+}
+
+int ssimu2_debug_read_tile_partials(ssimu2_t* h, uint64_t ticket, double* out, size_t out_doubles)
+{
+    if (!h || !out) return SSIMU2_E_INVALID;
+    if (!h->tile) return SSIMU2_E_UNSUPPORTED;
+    int r = ssimu2_wait(h, ticket);
+    if (r) return r;
+    DeviceGuard guard(h->cfg.device);
+    Slot* sl;
+    size_t idx;
+    if ((r = debug_slot(h, ticket, &sl, &idx))) return r;
+    const size_t n = h->tile_entries * 18;
+    if (out_doubles < n) return SSIMU2_E_INVALID;
+    CU_TRY(cudaMemcpy(out, sl->tiles + idx * n, n * sizeof(double), cudaMemcpyDeviceToHost));
+    return SSIMU2_OK;
+}
+
+int ssimu2_debug_tile_units(const ssimu2_t* h, uint32_t entry0[6], uint32_t units[6], uint32_t unit_cols[6])
+{
+    if (!h || !entry0 || !units || !unit_cols) return SSIMU2_E_INVALID;
+    if (!h->tile) return SSIMU2_E_UNSUPPORTED;
+    for (int s = 0; s < kMaxScales; s++) {
+        int u = 0;
+        const bool on = s < h->geo.nscales;
+        entry0[s] = on ? (uint32_t)tile_layout(h->geo, h->tile_log2, s, &u) : 0u;
+        units[s] = on ? (uint32_t)u : 0u;
+        unit_cols[s] = on ? std::min<uint32_t>(64u, h->tile >> s) : 0u;
+    }
     return SSIMU2_OK;
 }
 

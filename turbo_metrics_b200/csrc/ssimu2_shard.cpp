@@ -203,6 +203,7 @@ int ssimu2_shard_create_mixed(ssimu2_shard_t** out, const ssimu2_config* cfg, co
 {
     if (!out || !cfg || !devices || n_devices == 0 || n_devices > 64) return SSIMU2_E_INVALID;
     *out = nullptr;
+    if (cfg->tile) return SSIMU2_E_UNSUPPORTED;   // tile maps are per handle; the shard API returns scores only
     ssimu2_shard* s = new (std::nothrow) ssimu2_shard();
     if (!s) return SSIMU2_E_NOMEM;
     s->cfg = *cfg;

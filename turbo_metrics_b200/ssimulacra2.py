@@ -110,11 +110,11 @@ class DeviceFrame:
 
 
 def make_config(width, height, fmt, matrix=ColorMatrix.BT709, full_range=False, device=0, batch=0, ring=0,
-                pipeline=_lib.PIPELINE_DEFAULT, flags=0, input_group=0) -> Config:
+                pipeline=_lib.PIPELINE_DEFAULT, flags=0, input_group=0, tile=0) -> Config:
     cfg = Config()
     cfg.width, cfg.height, cfg.format, cfg.matrix = width, height, int(fmt), int(matrix)
     cfg.full_range, cfg.device, cfg.batch, cfg.ring = int(full_range), device, batch, ring
-    cfg.pipeline, cfg.flags, cfg.input_group = pipeline, flags, input_group
+    cfg.pipeline, cfg.flags, cfg.input_group, cfg.tile = pipeline, flags, input_group, tile
     return cfg
 
 
@@ -164,7 +164,8 @@ class Ssimulacra2:
                  batch: int = 0, ring: int = 0, pipeline: Optional[str] = None, score_only: bool = False,
                  input_group: int = 0, timing: bool = True, p016_deep: bool = False, dis_fmt: Optional[PixelFormat] = None,
                  dis_matrix: Optional[ColorMatrix] = None, dis_full_range: Optional[bool] = None,
-                 dis_p016_deep: Optional[bool] = None, dis_width: Optional[int] = None, dis_height: Optional[int] = None):
+                 dis_p016_deep: Optional[bool] = None, dis_width: Optional[int] = None, dis_height: Optional[int] = None,
+                 tile: int = 0):
         """pipeline: None / "hv" = the product pipeline (front-end, fused H+V kernel, finalize); "split" = development
         pipeline with the H-pass planes in HBM (debug_read(what=1)).
         score_only: SSIMU2_FLAG_SCORE_ONLY -- skip the work whose weights are zero (scores identical, no norms).
@@ -176,14 +177,16 @@ class Ssimulacra2:
         side's own `nbytes`.
         dis_width, dis_height: the distorted frames' size when it is smaller than width x height (e.g. a 720p encode scored
         against its 1080p source): they are upscaled to width x height on the GPU (bicubic Catmull-Rom, ssimu2_source) and
-        scored there.  Distorted frames are then given at their own size."""
+        scored there.  Distorted frames are then given at their own size.
+        tile: per-tile scores on a grid of tile x tile pixels (a power of two, 64 .. 32768; 0 = off): get_tile_scores() gives
+        a SSIMULACRA2 score per tile, pooled from the frame's own error maps (ssimu2_config.tile)."""
         self._h = C.c_void_p()
         if pipeline not in (None, "hv", "split"):
             raise ValueError(f"unknown pipeline {pipeline!r}")
         flags = (_lib.FLAG_SCORE_ONLY if score_only else 0) | (0 if timing else _lib.FLAG_NO_TIMING) | \
                 (_lib.FLAG_P016_DEEP if p016_deep else 0)
         cfg = make_config(width, height, fmt, matrix, full_range, device, batch, ring,
-                          _lib.PIPELINE_SPLIT if pipeline == "split" else _lib.PIPELINE_DEFAULT, flags, input_group)
+                          _lib.PIPELINE_SPLIT if pipeline == "split" else _lib.PIPELINE_DEFAULT, flags, input_group, tile)
         src = make_source(cfg, dis_fmt, dis_matrix, dis_full_range, dis_p016_deep, dis_width, dis_height)
         if src is None:
             check(_lib.lib().ssimu2_create(C.byref(self._h), C.byref(cfg)), "ssimu2_create")
@@ -326,6 +329,22 @@ class Ssimulacra2:
               "ssimu2_get_norms")
         return out
 
+    def tile_grid(self):
+        """-> (tile, tiles_x, tiles_y, capacity): the tile size (0 without tiles), the grid, and how many of the most recent
+        tickets still have their tile map."""
+        t, x, y, cap = C.c_uint32(), C.c_uint32(), C.c_uint32(), C.c_uint64()
+        check(_lib.lib().ssimu2_get_tile_grid(self._h, C.byref(t), C.byref(x), C.byref(y), C.byref(cap)), "ssimu2_get_tile_grid")
+        return t.value, x.value, y.value, cap.value
+
+    def get_tile_scores(self, ticket: int) -> np.ndarray:
+        """The ticket's tile scores, float64 of shape (tiles_y, tiles_x): 100 where nothing differs, lower where it does."""
+        _, tx, ty, _ = self.tile_grid()
+        out = np.zeros((ty, tx), np.float64)
+        check(_lib.lib().ssimu2_get_tile_scores(self._h, ticket, out.ctypes.data_as(C.POINTER(C.c_double)), out.size),
+              "ssimu2_get_tile_scores")
+        self._release()
+        return out
+
     def compute_sync(self, ref: DeviceFrame, dis: DeviceFrame, stream=None) -> float:
         """`Ssimulacra2::compute_sync` (lib.rs:271-279)."""
         return self.get_score(self.compute(ref, dis, stream))
@@ -387,6 +406,25 @@ class Ssimulacra2:
         check(_lib.lib().ssimu2_debug_read_partials(self._h, ticket, out.ctypes.data_as(C.POINTER(C.c_double)), out.size),
               "ssimu2_debug_read_partials")
         return [out[s0:s0 + n] for s0, n in zip(strip0, n_strips)]
+
+    def debug_tile_units(self):
+        """-> per scale (entry0, units, unit_cols): where the scale starts in the tile table, its column units per tile row
+        and the columns of one unit."""
+        e0, un, uc = (C.c_uint32 * 6)(), (C.c_uint32 * 6)(), (C.c_uint32 * 6)()
+        check(_lib.lib().ssimu2_debug_tile_units(self._h, e0, un, uc), "ssimu2_debug_tile_units")
+        return [(e0[s], un[s], uc[s]) for s in range(self.info().nscales)]
+
+    def debug_tile_partials(self, ticket: int) -> list:
+        """The pair's per-tile sums, one float64 array of shape (tiles_y, units, 3, 6) per scale (entries as in
+        debug_partials; a unit is a tile column, or a 64-column strip of it).  Valid until the batch slot that served the
+        ticket is reused, like debug_read."""
+        layout = self.debug_tile_units()
+        _, _, ty, _ = self.tile_grid()
+        n = sum(ty * u for _, u, _ in layout)
+        out = np.zeros((n, 3, 6), np.float64)
+        check(_lib.lib().ssimu2_debug_read_tile_partials(self._h, ticket, out.ctypes.data_as(C.POINTER(C.c_double)), out.size),
+              "ssimu2_debug_read_tile_partials")
+        return [out[e0:e0 + ty * u].reshape(ty, u, 3, 6) for e0, u, _ in layout]
 
     def kernel_ms(self, reset: bool = False):
         """-> (ms_total[4] for frontend/hpass/vpass/finalize, batches, pairs) since the last reset."""
